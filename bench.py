@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5              # our engine (default)
     torchrun --nproc-per-node N ... bench.py --gpus N ...        # one rank per GPU, weak scaling (64 images / rank)
     python bench.py --impl reference --steps 3 --warmup 1       # reference arm: CPU fp32 forward on the host cores
+    python bench.py --steps 20 --dump-outputs DIR                # also write the last timed step's outputs to DIR
 
 A "step" is one forward of the path over one synthetic batch: configs[1] of BASELINE.json
 (bs=64 synthetic 256x256 inputs cropped to 256x192, ViT-H/16 + token decoder + SMPL, fp16 operands / fp32
@@ -215,6 +216,45 @@ def run_reference(args):
     }), flush=True)
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_MAX_ELEMS_PER_ARRAY = 4 << 20
+
+
+def clone_outputs(out: dict) -> dict:
+    """Device copy of a forward's output dict (the aliased buffers are overwritten by later forwards)."""
+    return {k: clone_outputs(v) if isinstance(v, dict) else v.clone() for k, v in out.items()}
+
+
+def dump_outputs(out: dict, directory: str) -> list:
+    """Writes every array of a forward's output dict as <directory>/<name>.npy in float32 (a nested dict's arrays as
+    <outer>.<inner>.npy), within DUMP_MAX_BYTES in all.  An array larger than its share of the budget (at this workload
+    only cls_logits_softmax: 64 x 160 x 2048) is written as a fixed sample of its flattened elements: the sorted indices
+    drawn by numpy's default_rng(0), the same in every run, so that two builds compare element for element."""
+    import numpy as np
+    flat = {}
+
+    def walk(prefix, d):
+        for k, v in d.items():
+            if isinstance(v, dict):
+                walk(f"{prefix}{k}.", v)
+            else:
+                flat[prefix + k] = v.detach().float().cpu().numpy()
+
+    walk("", out)
+    os.makedirs(directory, exist_ok=True)
+    left = (DUMP_MAX_BYTES - 4096 * len(flat)) // 4          # elements; 4 KB per file covers the .npy header
+    written = []
+    for i, (name, a) in enumerate(sorted(flat.items(), key=lambda kv: (kv[1].size, kv[0]))):
+        share = min(DUMP_MAX_ELEMS_PER_ARRAY, left // (len(flat) - i))
+        if a.size > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))]
+            name += ".sample"
+        np.save(os.path.join(directory, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+        left -= a.size
+        written.append(name)
+    return written
+
+
 # ---------------------------------------------------------------------------------------------------------
 def cuda_time(fn, n=5, warm=2):
     import torch
@@ -312,7 +352,16 @@ def main():
     ap.add_argument("--streams", type=int, default=0, choices=[0, 1, 2, 3, 4],
                     help="1: consecutive steps replay on one stream; n > 1: round-robin on n streams (n steps in flight, single "
                          "GPU only); 0 (default): measure 1 and 4 at N=1 and report the faster as `value`")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last step of the path `value` was measured on "
+                         "as DIR/<name>.npy (float32, at most 64 MB in all; see dump_outputs).  The one- and n-stream "
+                         "engines sum in different orders and their outputs differ slightly; --streams fixes which one "
+                         "is measured")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 engine's timed path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -377,10 +426,11 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_resident()
+        out_last = step_resident()
     e1.record()
     barrier()
     t_win1 = time.time()
+    last_outputs = {"serial": clone_outputs(out_last)} if args.dump_outputs and rank == 0 else None
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     ms_step = ms_total / args.steps
     value = world * B * 1e3 / ms_step
@@ -427,6 +477,8 @@ def main():
         e1.record(main)
         torch.cuda.synchronize()
         t_d1 = time.time()
+        if last_outputs is not None:
+            last_outputs["dual"] = clone_outputs(last[(args.steps - 1) % NS])
         ms_dual = e0.elapsed_time(e1) / args.steps
         dual = {"value": B * 1e3 / ms_dual, "ms_per_step": ms_dual, "streams": NS, "window": (t_d0, t_d1),
                 "max_abs_vertex_diff_vs_serial": dev_max,
@@ -437,6 +489,11 @@ def main():
                               "max_abs_vertex_diff_vs_serial": dev_max}), file=sys.stderr, flush=True)
     head = dual if (dual is not None and (args.streams > 1 or dual["value"] > serial["value"])) else serial
     value, ms_step_head = head["value"], head["ms_per_step"]
+    if last_outputs is not None:
+        names = dump_outputs(last_outputs["dual" if head is dual else "serial"], args.dump_outputs)
+        print(json.dumps({"dumped": names, "dir": args.dump_outputs, "steps_in_flight": head["streams"]}), file=sys.stderr,
+              flush=True)
+        del last_outputs
     clocks = None
     if rank == 0:
         time.sleep(0.12)

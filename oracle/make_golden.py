@@ -10,6 +10,7 @@ INFRASTRUCTURE ONLY.
 from __future__ import annotations
 
 import argparse
+import hashlib
 from pathlib import Path
 
 import numpy as np
@@ -209,6 +210,86 @@ def encoder_goldens(ns) -> None:
     print("wrote tok_encoder golden:", idx_a.unique().numel(), "/", idx_b.unique().numel(), "distinct codes")
 
 
+def _digest(a: np.ndarray) -> np.ndarray:
+    return np.array(hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest())
+
+
+def live_parity_goldens(ns) -> None:
+    """What the *_equals_live_reference tests compare the restatements with, from the LIVE reference on inputs other
+    than the goldens above.  Large arrays are kept as a fixed strided sample (a prime stride, so that every token and
+    channel is visited); the bit-exact pre-processing crops are kept as a sample plus the SHA-256 of the whole crop."""
+    from . import eval_oracle
+    # --- forward of the reference modules (tiny config, weights 99, SMPL 5, images 11, batch 3) and the hard quantiser
+    cfg = tiny_config(vit_depth=2)
+    sd, smpl = synth.make_state_dict(cfg, 99), synth.make_smpl(cfg, 5)
+    img = synth.make_images(3, cfg, 11)
+    out = ref_import.reference_forward(ns, ref_import.build_backbone(ns, sd, cfg), ref_import.build_head(ns, sd, cfg),
+                                       smpl, img, cfg)
+    cb, x = small_vq_inputs()
+    qz = ns.quantize_cnn.QuantizeEMAReset(64, 32)
+    qz.codebook = cb
+    with torch.no_grad():
+        idx = qz.quantize(x)
+    np.savez_compressed(
+        GOLDEN / "forward_tiny_d2_seed99.npz", meta=np.array([99, 5, 11, 3], np.int64), stride=127,
+        vit_tokens_flat=out["_vit_tokens"].flatten()[::127].numpy(),
+        cls_probs_flat=out["cls_logits_softmax"].flatten()[::127].numpy(),
+        cls_argmax=out["cls_logits_softmax"].argmax(-1).numpy().astype(np.int16),
+        **{k: out[k].numpy() for k in ("pred_cam", "pred_keypoints_3d", "pred_vertices", "pred_keypoints_2d")},
+        vq_idx=idx.numpy().astype(np.int16))
+    # --- Evaluator metrics and compute_similarity_transform (pose_utils.py) on two seeded batches
+    ev = ref_import.load_eval_modules()
+    kl = list(range(25, 39))
+    arrays = {}
+    for seed in (0, 5):
+        o, b = eval_oracle.synthetic_eval_batch(5, V=300, seed=seed)
+        e = ev.pose_utils.Evaluator(dataset_length=8, keypoint_list=kl, pelvis_ind=39,
+                                    metrics=['mode_re', 'mode_mpjpe', 'mode_pve'], dataset='3DPW-TEST')
+        e({k: v.clone() for k, v in o.items()}, {k: (v.clone() if torch.is_tensor(v) else v) for k, v in b.items()})
+        arrays.update({f"mpjpe_{seed}": e.mode_mpjpe[:5], f"re_{seed}": e.mode_re[:5], f"pve_{seed}": e.mode_pve[:5],
+                       f"similarity_{seed}": ev.pose_utils.compute_similarity_transform(
+                           o["pred_keypoints_3d"], b["keypoints_3d"][..., :3]).numpy()})
+    np.savez_compressed(GOLDEN / "evaluator_seeds.npz", keypoint_list=np.array(kl, np.int32), **arrays)
+    # --- ViTDetDataset items: boxes inside, across the border and larger than the frame, with and without BBOX_SHAPE
+    ds_mod = ref_import.load_dataset_modules()
+    frame, boxes = live_preproc_scene()
+    arrays = {}
+    for name, shape in (("shape", (192, 256)), ("noshape", None)):
+        ds = ds_mod.vitdet_dataset.ViTDetDataset(ref_import.dataset_cfg(bbox_shape=shape), frame, boxes)
+        items = [ds[i] for i in range(len(boxes))]
+        arrays.update({f"{name}_img_flat": np.stack([it["img"].ravel()[::251] for it in items]),
+                       f"{name}_img_sha256": np.stack([_digest(it["img"]) for it in items]),
+                       f"{name}_img_dtype": np.array(str(items[0]["img"].dtype)),
+                       f"{name}_box_center": np.stack([it["box_center"] for it in items]),
+                       f"{name}_box_size": np.array([it["box_size"] for it in items], np.float32)})
+    np.savez_compressed(GOLDEN / "preproc_live.npz", boxes=boxes, stride=251, **arrays)
+    # --- EncodeTokens (encoder seed 77, poses seed 4)
+    rcfg = release_config()
+    sd = synth.make_tokenizer_encoder_state_dict(rcfg, 77)
+    enc = ref_import.build_encode_tokens(ns, sd, rcfg)
+    x = torch.randn(3, rcfg.tok_joints, 6, generator=torch.Generator().manual_seed(4))
+    with torch.no_grad():
+        idx, lat = enc(x), enc.quantizer.preprocess(enc.encoder(x))
+    np.savez_compressed(GOLDEN / "tok_encoder_seed77.npz", meta=np.array([77, 4, 3], np.int64), stride=31,
+                        idx=idx.numpy().astype(np.int32), latent_flat=lat.flatten()[::31].numpy())
+    print("wrote live parity goldens")
+
+
+def small_vq_inputs():
+    """A 64 x 32 codebook and 500 queries (seed 13)."""
+    g = torch.Generator().manual_seed(13)
+    return torch.randn(64, 32, generator=g), torch.randn(500, 32, generator=g)
+
+
+def live_preproc_scene():
+    """Random 300 x 420 BGR frame and four boxes (inside, across the border, up to the far corner, larger than the frame:
+    the last one takes the anti-alias blur)."""
+    rng = np.random.default_rng(9)
+    frame = rng.integers(0, 256, (300, 420, 3), dtype=np.uint8)
+    boxes = np.float32([[30.5, 20.25, 200.0, 280.0], [-50, -60, 180, 200], [100, 50, 419, 299], [-400, -300, 800, 700]])
+    return frame, boxes
+
+
 def rodrigues_goldens(ns) -> None:
     """Axis-angle -> rotation matrix by the reference's OWN two implementations (geometry.aa_to_rotmat, via a quaternion,
     geometry.py:5-46; rotation_utils.axis_angle_to_matrix, rotation_utils.py:411-443).  smplx's batch_rodrigues is not in
@@ -268,6 +349,9 @@ def main() -> None:
     if args.only == "vq":
         vq_large_golden(ref_import.load_modules())
         return
+    if args.only == "parity":
+        live_parity_goldens(ref_import.load_modules())
+        return
     if args.only == "forward":
         ns = ref_import.load_modules()
         forward_golden(ns, tiny_config(vit_depth=2), 2, "forward_tiny_d2.npz")
@@ -282,6 +366,7 @@ def main() -> None:
     preproc_goldens()
     encoder_goldens(ns)
     rodrigues_goldens(ns)
+    live_parity_goldens(ns)
     forward_golden(ns, tiny_config(vit_depth=2), 2, "forward_tiny_d2.npz")
     if args.release:
         forward_golden(ns, release_config(), 2, "forward_release_d32.npz")

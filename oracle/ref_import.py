@@ -8,9 +8,9 @@ import fine once
   * `timm.models.layers` is shimmed (only import of timm: backbones/vit.py:10),
   * `smplx` is stubbed (import-time body-model load in tokenization/models/vanilla_pose_vqvae.py:10-17),
   * torch.Tensor.cuda is neutralised on a CPU-only host (quantize_cnn.py:18 hard-codes .cuda()).
-Nothing is copied: the modules execute from /root/reference where they lie.  This file is used by
-oracle/make_golden.py (writes tests/golden/*.npz) and by tests that validate the restatement against
-the live reference; it is never reachable on the GPU box (no /root/reference there).
+Nothing is copied: the modules execute from the reference tree where they lie.  This file is used by
+oracle/make_golden.py, which writes tests/golden/*.npz; the tests compare with those files and never need
+the reference tree.
 """
 from __future__ import annotations
 
@@ -31,7 +31,11 @@ REF_ROOT = Path(os.environ.get("TOKENHMR_REFERENCE", "/root/reference"))
 
 
 def available() -> bool:
-    return (REF_ROOT / "tokenhmr" / "lib" / "models" / "backbones" / "vit.py").exists()
+    """True when the reference tree is present and readable (a tree the user may not enter counts as absent)."""
+    try:
+        return (REF_ROOT / "tokenhmr" / "lib" / "models" / "backbones" / "vit.py").is_file()
+    except OSError:
+        return False
 
 
 def _namespace(name: str, path: Path) -> None:

@@ -12,8 +12,7 @@ Pinning status
   * ViT, decoder, token classifier, tokenizer decoder, quantizer, rot6d, projection: PINNED against the
     reference's own modules executed in the build container (oracle/ref_import.py imports them file by
     file; oracle/make_golden.py stores their outputs under tests/golden/; tests/test_oracle_pinned.py
-    checks this restatement against those goldens, and against the live modules when /root/reference
-    exists).
+    checks this restatement against those goldens).
   * SMPL (smplx==0.1.28 lbs / SMPLLayer / VertexJointSelector): third-party, absent from /root/reference
     and not installable offline -> restated from the published algorithm (oracle/smpl_oracle.py),
     anchored on the reference call sites only: PARITY UNPINNED for that stage.

@@ -1,13 +1,14 @@
 """Input pre-processing (SURVEY §8 row f2).  CPU part: pins oracle/preproc_oracle.py against the golden items the
-LIVE reference ViTDetDataset produced, against cv2 / scipy themselves and against the live class; checks the C-ABI
+LIVE reference ViTDetDataset produced (two scenes) and against cv2 / scipy themselves; checks the C-ABI
 host planner (no CUDA call) bit for bit.  GPU part: thmr_preprocess_boxes vs the oracle and the goldens."""
+import hashlib
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import preproc_oracle as P
-from oracle import ref_import
-from oracle.make_golden import preproc_scene
+from oracle.make_golden import live_preproc_scene, preproc_scene
 
 MEAN = 255.0 * np.array(P.DEFAULT_MEAN)
 STD = 255.0 * np.array(P.DEFAULT_STD)
@@ -56,19 +57,20 @@ def test_oracle_pieces_match_cv2_and_scipy():
         np.testing.assert_allclose(P.gaussian_blur(img, sigma), want, rtol=0, atol=1e-12)
 
 
-def test_oracle_equals_live_reference_dataset():
-    if not ref_import.available():
-        pytest.skip("reference tree not present (GPU box)")
-    ds_mod = ref_import.load_dataset_modules()
-    rng = np.random.default_rng(9)
-    img = rng.integers(0, 256, (300, 420, 3), dtype=np.uint8)
-    boxes = np.float32([[30.5, 20.25, 200.0, 280.0], [-50, -60, 180, 200], [100, 50, 419, 299], [-400, -300, 800, 700]])
-    for shape in ((192, 256), None):
-        ds = ds_mod.vitdet_dataset.ViTDetDataset(ref_import.dataset_cfg(bbox_shape=shape), img, boxes)
+def test_oracle_equals_live_reference_dataset(golden_dir):
+    """Every crop equals the reference ViTDetDataset's bit for bit: a strided sample is compared value by value, the whole
+    crop through its SHA-256."""
+    g = np.load(golden_dir / "preproc_live.npz")
+    img, boxes = live_preproc_scene()
+    assert np.array_equal(boxes, g["boxes"])
+    stride = int(g["stride"])
+    for name, shape in (("shape", (192, 256)), ("noshape", None)):
         for i in range(len(boxes)):
-            ref, it = ds[i], P.vitdet_item(img, boxes[i], bbox_shape=shape)
-            assert np.array_equal(ref["img"], it["img"])
-            assert np.array_equal(ref["box_center"], it["box_center"]) and ref["box_size"] == it["box_size"]
+            it = P.vitdet_item(img, boxes[i], bbox_shape=shape)
+            assert str(it["img"].dtype) == str(g[f"{name}_img_dtype"])
+            assert np.array_equal(it["img"].ravel()[::stride], g[f"{name}_img_flat"][i]), f"{name} box {i}"
+            assert hashlib.sha256(np.ascontiguousarray(it["img"]).tobytes()).hexdigest() == g[f"{name}_img_sha256"][i]
+            assert np.array_equal(it["box_center"], g[f"{name}_box_center"][i]) and it["box_size"] == g[f"{name}_box_size"][i]
 
 
 # ------------------------------------------------------------------------------------------------ host planner
