@@ -1,4 +1,4 @@
-import torch, os, subprocess, time, threading
+import torch, subprocess, time, threading
 from tokenhmr_b200._lib import lib, check
 L = lib(); dev = torch.device("cuda:0"); torch.manual_seed(0)
 st = lambda: torch.cuda.current_stream().cuda_stream
@@ -24,7 +24,6 @@ def sample(fn, secs=2.5):
     vals = [tuple(float(x) for x in r.split(",")) for r in rows[n0+3:]]
     clk = sorted(v[0] for v in vals); pw = sorted(v[1] for v in vals)
     return ms, clk[len(clk)//2] if clk else 0, pw[len(pw)//2] if pw else 0
-print("DBG", os.environ.get("THMR_GEMM_DBG"))
 for name, fn in [("cublas", lambda: torch.matmul(A, B.t())), ("mine bn256", lambda: mine(256)), ("mine 2cta", lambda: mine(512))]:
     ms, clk, pw = sample(fn)
     print(f"{name}: {ms*1e3:.1f} us  {2*M*N*K/ms/1e9:.0f} TF  sm_clk {clk:.0f} MHz  power {pw:.0f} W  -> util {2*M*N*K/ms/1e9/(148*8192*clk*1e-6)*100:.0f}%", flush=True)

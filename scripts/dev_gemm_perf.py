@@ -16,7 +16,6 @@ def timeit(fn, iters=50):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / iters
 M = 12288
-print("THMR_GEMM_DBG =", os.environ.get("THMR_GEMM_DBG"))
 for (name, N, K, act, mode) in [("qkv", 3840, 1280, 0, "s16"), ("proj", 1280, 1280, 0, "add"), ("fc1", 5120, 1280, 1, "s16"), ("fc2", 1280, 5120, 0, "add")]:
     A = torch.randn(M, K, device=dev).half(); B = (torch.randn(N, K, device=dev) * 0.03).half()
     bias = torch.randn(N, device=dev)

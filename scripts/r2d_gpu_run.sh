@@ -1,5 +1,5 @@
 #!/bin/bash
-# Evidence call with the final defaults: whole GPU suite, VQ / LBS stand-alone timings (row-fastest tile order on and off),
+# Evidence call with the final defaults: whole GPU suite, VQ / LBS stand-alone timings,
 # the bench line (1 stream vs 4 streams), smoke(), ncu --set full of the SMPL blend GEMM and the skinning kernel.
 cd "${GRAFT_REPO_ROOT:-/root/repo}"
 export PYTHONPATH=.
@@ -10,7 +10,6 @@ el() { echo "[t+$(( $(date +%s) - T0 ))s] $*"; }
 timeout 400 python -m pytest tests -m gpu -q > $O/r2d_pytest_gpu.log 2>&1
 el "full pytest rc=$?"; tail -4 $O/r2d_pytest_gpu.log
 timeout 120 python scripts/dev_vq_lbs.py > $O/r2d_vq_lbs.log 2>&1; el "vq/lbs rc=$?"; cat $O/r2d_vq_lbs.log
-THMR_GEMM_MFAST=0 timeout 120 python scripts/dev_vq_lbs.py lbs > $O/r2d_lbs_nfast.log 2>&1; el "lbs column-fastest rc=$?"; cat $O/r2d_lbs_nfast.log
 timeout 420 python bench.py --steps 20 --warmup 5 > $O/r2d_bench_b200_n1.json 2> $O/r2d_bench_b200_n1.err
 el "bench rc=$?"; grep early $O/r2d_bench_b200_n1.err | head -3
 timeout 120 python -c "import __graft_entry__ as g; g.smoke()" > $O/r2d_smoke.log 2>&1

@@ -87,6 +87,15 @@ def test_product_never_imports_the_oracle():
         assert "import oracle" not in src and "from oracle" not in src, f
 
 
+def test_library_reads_only_the_known_environment_variables():
+    """Every getenv() of the native library selects something a caller relies on: THMR_VQ_SCREEN and THMR_SKIN_THREADS
+    pick between two timed schedules, THMR_NCCL_LIB locates a library.  A new switch has to be added here on purpose."""
+    names = set()
+    for f in sorted((ROOT / "tokenhmr_b200" / "csrc").glob("*.cu*")):
+        names.update(re.findall(r'getenv\(\s*"([^"]+)"', f.read_text()))
+    assert names == {"THMR_VQ_SCREEN", "THMR_SKIN_THREADS", "THMR_NCCL_LIB"}
+
+
 def test_vq_workspace_covers_both_schedules(built_lib):
     """thmr_vq_workspace_bytes is pure arithmetic (no CUDA call): it covers BOTH schedules of thmr_vq_argmin (the single exact
     pass needs a Q x 3D fp16 split operand; the screened one a 131072-row fp16 chunk, a 262144-row exact-pass round and the row

@@ -26,8 +26,6 @@
 //   warps 0..3 : softmax group 0 (TMEM lane quarter = warp id)      warp 8     : TMA producer
 //   warps 4..7 : softmax group 1                                     warps 9,10 : MMA issuers of chains 0,1 (9 owns TMEM)
 #pragma once
-#include <stdlib.h>
-
 #include "attention_common.cuh"
 
 namespace thmr {
@@ -41,22 +39,8 @@ constexpr int kAtt3Threads = 352;
 constexpr uint32_t kAtt3BufCols = 192;                            // TMEM columns per chain
 constexpr uint32_t kAtt3ColO = 96;
 
-// exp2 on the FMA pipe (Cody-Waite split + cubic, max rel. error 7.5e-5 on top of the fp16 rounding of P, 4.9e-4):
-// takes a share of the exponentials off the 16-lane/clk exp unit, the binding pipe of this kernel.  x <= ~0.
-__device__ __forceinline__ float poly_exp2(float x) {
-  x = fmaxf(x, -120.f);
-  const float r = x + 12582912.f;              // 1.5 * 2^23: round(x) lands in the low mantissa bits
-  const float f = x - (r - 12582912.f);        // [-0.5, 0.5]
-  float pl = fmaf(5.517164753e-02f, f, 2.426111206e-01f);
-  pl = fmaf(pl, f, 6.932609894e-01f);
-  pl = fmaf(pl, f, 9.999280737e-01f);
-  return __int_as_float(__float_as_int(pl) + (__float_as_int(r) << 23));
-}
-
-// Softmax pass 2 of one row: exp2(s * scale - mo) over 192 keys streamed from TMEM (one 32-column load ahead),
-// P as fp16 pairs written in place over consumed columns; returns the fp32 row sum.
-// POLY: 0 = all on the exp unit, 1 = every 4th element on the FMA pipe, 2 = every 2nd.
-template <int POLY>
+// 32 keys of softmax pass 2: exp2(s * scale - mo), accumulated into four partial row sums and written to TMEM as 16
+// fp16 pairs.
 __device__ __forceinline__ void att3_exp_chunk(const uint32_t (&cur)[32], uint32_t taddr, float sc, float mo,
                                                float& s0, float& s1, float& s2, float& s3) {
   uint32_t w16[16];
@@ -67,9 +51,9 @@ __device__ __forceinline__ void att3_exp_chunk(const uint32_t (&cur)[32], uint32
     const float x2 = fmaf(__uint_as_float(cur[e + 2]), sc, -mo);
     const float x3 = fmaf(__uint_as_float(cur[e + 3]), sc, -mo);
     const float e0 = fast_exp2(x0);
-    const float e1 = POLY >= 2 ? poly_exp2(x1) : fast_exp2(x1);
+    const float e1 = fast_exp2(x1);
     const float e2 = fast_exp2(x2);
-    const float e3 = POLY >= 1 ? poly_exp2(x3) : fast_exp2(x3);
+    const float e3 = fast_exp2(x3);
     s0 += e0; s1 += e1; s2 += e2; s3 += e3;
     __half2 h01 = __floats2half2_rn(e0, e1);
     __half2 h23 = __floats2half2_rn(e2, e3);
@@ -84,8 +68,6 @@ __device__ __forceinline__ void att3_exp_chunk(const uint32_t (&cur)[32], uint32
 // behind the columns already read); returns the fp32 row sum.
 // The loops are deliberately NOT fully unrolled: the straight-line version of this kernel was ~100 KB of SASS and the
 // softmax warps spent 40-50 % of their samples in stall_no_inst (instruction fetch).
-// POLY: 0 = all on the exp unit, 1 = every 4th element on the FMA pipe, 2 = every 2nd.
-template <int POLY>
 __device__ __forceinline__ float att3_pass2(uint32_t tb, float sc, float mo) {
   uint32_t va[32], vb[32];
   float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
@@ -94,10 +76,10 @@ __device__ __forceinline__ float att3_pass2(uint32_t tb, float sc, float mo) {
   for (int jj = 0; jj < 3; ++jj) {
     tmem_ld_x32(tb + (2 * jj + 1) * 32, vb);
     tmem_ld_wait();
-    att3_exp_chunk<POLY>(va, tb + (2 * jj) * 16, sc, mo, s0, s1, s2, s3);
+    att3_exp_chunk(va, tb + (2 * jj) * 16, sc, mo, s0, s1, s2, s3);
     if (jj < 2) tmem_ld_x32(tb + (2 * jj + 2) * 32, va);
     tmem_ld_wait();
-    att3_exp_chunk<POLY>(vb, tb + (2 * jj + 1) * 16, sc, mo, s0, s1, s2, s3);
+    att3_exp_chunk(vb, tb + (2 * jj + 1) * 16, sc, mo, s0, s1, s2, s3);
   }
   tmem_st_wait();
   return (s0 + s1) + (s2 + s3);
@@ -137,7 +119,7 @@ __device__ __forceinline__ float att3_pass1(uint32_t tb, float* dbg_row) {
   return fmaxf(fmaxf(m0, m1), fmaxf(m2, m3));
 }
 
-template <int POLY, bool DBG>
+template <bool DBG>
 __global__ void __launch_bounds__(kAtt3Threads, 1)
 vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_constant__ CUtensorMap tmQK64,
                       const __grid_constant__ CUtensorMap tmQK16, const __grid_constant__ CUtensorMap tmO,
@@ -158,16 +140,12 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const bool dup_alt = !(p.p_in_tmem & 1);     // experiment knobs (THMR_ATTN_TS): bit 0 = fixed duplicate rows
-  const bool use_turns = !(p.p_in_tmem & 8);   // bit 3 = no exp-phase alternation between the chains
   // Q and K arrive as one [192 x 64] SWIZZLE_128B box (dims 0..63: four of the five 16-wide UMMA k-chunks) plus one
   // [192 x 16] SWIZZLE_32B box: 384 TMA row requests per matrix instead of the 960 32-byte requests of five chunk boxes
-  // (the MMA issuers spent 15 % of the kernel waiting for the next head's Q, K).  Bit 5 = the round-1 five-chunk layout.
-  const bool wide_qk = !(p.p_in_tmem & 32);
+  // (the MMA issuers spent 15 % of the kernel waiting for the next head's Q, K).  V keeps the five-chunk 3-D view.
   const int nheads = (p.num_problems - static_cast<int>(blockIdx.x) + static_cast<int>(gridDim.x) - 1) /
                      static_cast<int>(gridDim.x);
 
-  pdl_launch_dependents();
   stamp_start(p.stamp);
   if (warp == 8 && lane == 0) {
     tma_prefetch_desc(&tmQKV);
@@ -195,15 +173,11 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();       // Q, K, V are the predecessor's output
 
   if (warp == 8) {
     // ---------------------------------------------------------------- TMA producers: lane 0 streams Q,K, lane 1 streams V
     // (two threads so that a V stage still held by the PV MMAs never delays the next Q,K load)
     if (lane < 2) {
-      // bit 4 of the knobs (THMR_L2_HINTS & 2): Q, K, V are dead once this kernel has read them -> evict_first
-      const bool hint = (p.p_in_tmem & 16) != 0;
-      const uint64_t pol = l2_policy_evict_first();
       for (int i = 0; i < nheads; ++i) {
         const int prob = blockIdx.x + i * gridDim.x;
         const int b = prob / p.heads, h = prob % p.heads;
@@ -213,24 +187,15 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
         if (lane == 0) {
           mbar_wait(&qk_empty[st], ph ^ 1);
           mbar_arrive_expect_tx(&qk_full[st], 2 * kAttMatBytes);
-          if (wide_qk) {
-            const int cq = h * kAttHeadDim, ck = (p.heads + h) * kAttHeadDim;
-            tma_load_2d(sQ, &tmQK64, &qk_full[st], cq, b * kAttTokens);
-            tma_load_2d(sQ + kAttWideBytes, &tmQK16, &qk_full[st], cq + 64, b * kAttTokens);
-            tma_load_2d(sQ + kAttMatBytes, &tmQK64, &qk_full[st], ck, b * kAttTokens);
-            tma_load_2d(sQ + kAttMatBytes + kAttWideBytes, &tmQK16, &qk_full[st], ck + 64, b * kAttTokens);
-          } else if (hint) {
-            tma_load_3d_hint(sQ, &tmQKV, &qk_full[st], 0, b * kAttTokens, h * kAttChunks, pol);
-            tma_load_3d_hint(sQ + kAttMatBytes, &tmQKV, &qk_full[st], 0, b * kAttTokens, (p.heads + h) * kAttChunks, pol);
-          } else {
-            tma_load_3d(sQ, &tmQKV, &qk_full[st], 0, b * kAttTokens, h * kAttChunks);
-            tma_load_3d(sQ + kAttMatBytes, &tmQKV, &qk_full[st], 0, b * kAttTokens, (p.heads + h) * kAttChunks);
-          }
+          const int cq = h * kAttHeadDim, ck = (p.heads + h) * kAttHeadDim;
+          tma_load_2d(sQ, &tmQK64, &qk_full[st], cq, b * kAttTokens);
+          tma_load_2d(sQ + kAttWideBytes, &tmQK16, &qk_full[st], cq + 64, b * kAttTokens);
+          tma_load_2d(sQ + kAttMatBytes, &tmQK64, &qk_full[st], ck, b * kAttTokens);
+          tma_load_2d(sQ + kAttMatBytes + kAttWideBytes, &tmQK16, &qk_full[st], ck + 64, b * kAttTokens);
         } else {
           mbar_wait(&v_empty[st], ph ^ 1);
           mbar_arrive_expect_tx(&v_full[st], kAttMatBytes);
-          if (hint) tma_load_3d_hint(sQ + 2 * kAttMatBytes, &tmQKV, &v_full[st], 0, b * kAttTokens, (2 * p.heads + h) * kAttChunks, pol);
-          else tma_load_3d(sQ + 2 * kAttMatBytes, &tmQKV, &v_full[st], 0, b * kAttTokens, (2 * p.heads + h) * kAttChunks);
+          tma_load_3d(sQ + 2 * kAttMatBytes, &tmQKV, &v_full[st], 0, b * kAttTokens, (2 * p.heads + h) * kAttChunks);
         }
       }
     }
@@ -245,34 +210,25 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
       constexpr uint32_t idesc_o = make_idesc_f16(128, kAttHeadDim, 0, 1);     // P V   : V is N-major
       const uint32_t smem_a = smem_u32(smem);
       const uint32_t tb = __shfl_sync(0xffffffffu, tmem_base, 0) + g * kAtt3BufCols;
-      long long w_oe = 0, w_qk = 0, w_p = 0, w_v = 0;
-      const long long t_begin = clock64();
       for (int i = 0; i < nheads; ++i) {
         const int st = i & 1;
         const uint32_t ph = (i >> 1) & 1;
         const uint32_t sQ = smem_a + st * kAtt3StageBytes;
         const int t = ((i & 1) == g) ? 0 : 1;
-        const int row0 = t ? ((dup_alt && ((i >> 1) & 1)) ? 128 : 64) : 0;
-        long long t0 = clock64();
+        const int row0 = t ? (((i >> 1) & 1) ? 128 : 64) : 0;
         mbar_wait(&o_empty[g], (i & 1) ^ 1);     // the chain's previous tile has drained
-        long long t1 = clock64();
-        w_oe += t1 - t0;
         mbar_wait(&qk_full[st], ph);
-        w_qk += clock64() - t1;
         tc_fence_after();
         if (elect_one()) {
 #pragma unroll
           for (int kc = 0; kc < kAttChunks; ++kc) {
             uint64_t da, db;
-            if (wide_qk && kc < 4) {           // k-chunk kc = bytes [32 kc, 32 kc + 32) of the 128-byte rows
+            if (kc < 4) {           // k-chunk kc = bytes [32 kc, 32 kc + 32) of the 128-byte rows
               da = make_smem_desc(sQ + row0 * 128 + kc * 32, 16, 1024, kSwz128);
               db = make_smem_desc(sQ + kAttMatBytes + kc * 32, 16, 1024, kSwz128);
-            } else if (wide_qk) {
+            } else {
               da = make_smem_desc(sQ + kAttWideBytes + row0 * 32, 16, 256, kSwz32);
               db = make_smem_desc(sQ + kAttMatBytes + kAttWideBytes, 16, 256, kSwz32);
-            } else {
-              da = make_smem_desc(sQ + kc * kAttChunkBytes + row0 * 32, 16, 256, kSwz32);
-              db = make_smem_desc(sQ + kAttMatBytes + kc * kAttChunkBytes, 16, 256, kSwz32);
             }
             umma_f16_ss(tb, da, db, idesc_s, kc != 0);
           }
@@ -280,12 +236,8 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
           umma_commit(&qk_empty[st]);
         }
         __syncwarp();
-        t0 = clock64();
         mbar_wait(&p_full[g], i & 1);
-        t1 = clock64();
-        w_p += t1 - t0;
         mbar_wait(&v_full[st], ph);
-        w_v += clock64() - t1;
         tc_fence_after();
         const uint32_t sV = sQ + 2 * kAttMatBytes;
         // (splitting these into two halves that start under the second half of the exponentials is not possible: O
@@ -301,12 +253,6 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
         }
         __syncwarp();
       }
-      if (p.dbg_counters && lane == 0) {
-        unsigned long long* c = p.dbg_counters + blockIdx.x * 32;
-        c[g ? 8 : 0] = clock64() - t_begin;
-        c[g ? 15 : 1] = w_oe;
-        c[16 + 3 * g] = w_qk; c[17 + 3 * g] = w_p; c[18 + 3 * g] = w_v;
-      }
     }
   } else {
     // ------------------------------------------------------------------ softmax + epilogue groups
@@ -315,56 +261,41 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
     const int trow = q * 32 + lane;          // row inside the 128-row tile == TMEM lane
     const uint32_t tb = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + g * kAtt3BufCols;
     uint8_t* stage_out = smem + kAtt3OffOut + warp * kAtt3OutWarpBytes;
-    long long w_s = 0, w_o = 0, c_p1 = 0, c_p2 = 0, c_epi = 0, w_turn = 0;
-    const long long t_begin = clock64();
     for (int i = 0; i < nheads; ++i) {
       const int prob = blockIdx.x + i * gridDim.x;
       const int b = prob / p.heads, h = prob % p.heads;
       const int t = ((i & 1) == g) ? 0 : 1;
-      const bool low = dup_alt && ((i >> 1) & 1);            // tile 1 = rows 128..255, useful lanes 0..63
+      const bool low = (i >> 1) & 1;            // tile 1 = rows 128..255, useful lanes 0..63
       const bool active = (t == 0) || (low ? q < 2 : q >= 2);
       const int row0 = t ? (low ? 128 : 64) : 0;
-      long long t0 = clock64();
       if (lane == 0) mbar_wait(&s_full[g], i & 1);
       __syncwarp();
       tc_fence_after();
-      long long t1 = clock64();
-      w_s += t1 - t0;
       float sum = 0.f;
       float mo = 0.f;
       if (active) {
         // ---- pass 1: row maximum
         float* dbg_row = DBG ? p.dbg_s + (static_cast<size_t>(prob) * kAttTokens + row0 + trow) * kAttTokens : nullptr;
         mo = att3_pass1<DBG>(tb, dbg_row) * p.scale_log2e;
-        c_p1 += clock64() - t1;
       }
       // the exp unit belongs to one warp of the sub-partition at a time: two chains left alone run in lock-step
       // (both exponentiate, then both queue for the tensor pipe), which serialises everything again
-      if (use_turns) {
-        const long long tt = clock64();
-        if (lane == 0) mbar_wait(&turn[g * 4 + q], g ? (i & 1) : ((i & 1) ^ 1));
-        __syncwarp();
-        w_turn += clock64() - tt;
-      }
+      if (lane == 0) mbar_wait(&turn[g * 4 + q], g ? (i & 1) : ((i & 1) ^ 1));
+      __syncwarp();
       if (active) {
-        const long long t2 = clock64();
         // ---- pass 2: exponentials, row sum, P (fp16) in place over the consumed S columns
-        sum = att3_pass2<POLY>(tb, p.scale_log2e, mo);
-        c_p2 += clock64() - t2;
+        sum = att3_pass2(tb, p.scale_log2e, mo);
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
-        if (use_turns) mbar_arrive(&turn[(g ^ 1) * 4 + q]);
+        mbar_arrive(&turn[(g ^ 1) * 4 + q]);
         mbar_arrive(&p_full[g]);
       }
       // ---- epilogue of this tile
-      t0 = clock64();
       if (lane == 0) mbar_wait(&o_full[g], i & 1);
       __syncwarp();
       tc_fence_after();
-      t1 = clock64();
-      w_o += t1 - t0;
       if (active) {
         uint32_t o0[32], o1[32], o2[16];
         tmem_ld_x32(tb + kAtt3ColO, o0);
@@ -407,7 +338,6 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
           tma_store_2d(&tmO, stage_out, h * kAttHeadDim, b * kAttTokens + row0 + q * 32);
           tma_store_commit();
         }
-        c_epi += clock64() - t1;
       } else {
         tc_fence_before();
         __syncwarp();
@@ -415,11 +345,6 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
       }
     }
     if (lane == 0) tma_store_wait_read<0>();
-    if (p.dbg_counters && lane == 0 && (warp == 2 || warp == 6)) {
-      unsigned long long* c = p.dbg_counters + blockIdx.x * 32 + (g ? 9 : 2);
-      c[0] = clock64() - t_begin; c[1] = w_s; c[2] = w_o; c[3] = c_p1; c[4] = c_p2; c[5] = c_epi;
-      p.dbg_counters[blockIdx.x * 32 + 22 + g] = w_turn;
-    }
   }
 
   tc_fence_before();
@@ -430,27 +355,22 @@ vit_attention3_kernel(const __grid_constant__ CUtensorMap tmQKV, const __grid_co
   }
 }
 
-template <int POLY, bool DBG>
+template <bool DBG>
 inline int attention3_launch_t(const AttnPlan& plan, cudaStream_t st) {
   static bool configured = false;
   if (!configured) {
-    THMR_CUDA(cudaFuncSetAttribute(vit_attention3_kernel<POLY, DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    THMR_CUDA(cudaFuncSetAttribute(vit_attention3_kernel<DBG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    kAtt3SmemBytes));
     configured = true;
   }
-  THMR_CUDA(launch_pdl(vit_attention3_kernel<POLY, DBG>, plan.grid, kAtt3Threads, kAtt3SmemBytes, st, plan.tm, plan.tm_qk64,
-                       plan.tm_qk16, plan.tm_out, plan.p));
+  vit_attention3_kernel<DBG><<<plan.grid, kAtt3Threads, kAtt3SmemBytes, st>>>(plan.tm, plan.tm_qk64, plan.tm_qk16,
+                                                                              plan.tm_out, plan.p);
+  THMR_CUDA(cudaGetLastError());
   return THMR_OK;
 }
 
-// knobs (THMR_ATTN_TS): bits 1-2 = share of exponentials computed on the FMA pipe (0, 1/4, 1/2)
 inline int attention3_launch(const AttnPlan& plan, cudaStream_t st) {
-  if (plan.p.dbg_s) return attention3_launch_t<0, true>(plan, st);
-  switch ((plan.p.p_in_tmem >> 1) & 3) {
-    case 1: return attention3_launch_t<1, false>(plan, st);
-    case 2: return attention3_launch_t<2, false>(plan, st);
-    default: return attention3_launch_t<0, false>(plan, st);
-  }
+  return plan.p.dbg_s ? attention3_launch_t<true>(plan, st) : attention3_launch_t<false>(plan, st);
 }
 
 inline int attention_dispatch(const AttnPlan& plan, cudaStream_t st) { return attention3_launch(plan, st); }

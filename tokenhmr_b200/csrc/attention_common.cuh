@@ -4,8 +4,6 @@
 // the first two generations (P through shared memory; single chain with P in TMEM) were removed in round 2 after losing
 // their A/B (round-1 numbers: DESIGN.md section 9).
 #pragma once
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -25,9 +23,7 @@ struct AttnParams {
   __half* out;       // [B*192, ldo], head h at columns [80 h, 80 h + 80)
   int ldo;
   float* dbg_s;      // optional [B*H, 192, 192] raw scores (tests only)
-  unsigned long long* dbg_counters;  // optional [gridDim.x][16] cycle counters (THMR_ATTN_COUNTERS)
   unsigned long long* stamp;   // in-graph start stamp (nullable)
-  int p_in_tmem;     // experiment knobs (THMR_ATTN_TS bits, see attention3_tcgen05.cuh); bit 4 = Q/K/V loaded evict_first
 };
 
 __device__ __forceinline__ float fast_exp2(float x) {
@@ -58,7 +54,7 @@ inline int make_tmap_qkv(CUtensorMap* out, const void* qkv, uint64_t rows, uint6
 struct AttnPlan {
   CUtensorMap tm_qk64;  // Q / K: [192 rows x 64 columns] boxes, 128-byte rows, SWIZZLE_128B (dims 0..63 of a head)
   CUtensorMap tm_qk16;  // Q / K: [192 rows x 16 columns] boxes, SWIZZLE_32B (dims 64..79)
-  CUtensorMap tm;
+  CUtensorMap tm;       // V: the 3-D five-chunk view (make_tmap_qkv)
   CUtensorMap tm_out;   // [B*192, H*80] fp16 output, 32-row x 80-column boxes (third-generation kernel)
   AttnParams p;
   int grid;
@@ -83,9 +79,6 @@ inline int attention_make_plan(const __half* qkv, int ld_qkv, int B, int heads, 
   plan->p.ldo = ldo;
   plan->p.dbg_s = dbg_s;
   plan->p.stamp = nullptr;
-  { const char* e = getenv("THMR_ATTN_TS"); plan->p.p_in_tmem = e ? atoi(e) : 0; }
-  { const char* e = getenv("THMR_L2_HINTS"); if (e && (atoi(e) & 2)) plan->p.p_in_tmem |= 16; }
-  { const char* e = getenv("THMR_ATTN_COUNTERS"); plan->p.dbg_counters = e ? reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0)) : nullptr; }
   plan->grid = plan->p.num_problems < num_sms() ? plan->p.num_problems : num_sms();
   return THMR_OK;
 }

@@ -101,14 +101,6 @@ struct Bump {
   }
 };
 
-// Programmatic dependent launch (THMR_PDL=1, off by default): a kernel launched through launch_pdl() may be scheduled
-// while its predecessor in the stream is still running; it must execute pdl_wait() before it touches anything the
-// predecessor reads or writes.  Every kernel launched this way calls pdl_launch_dependents() first, so that its own
-// successor can be placed on SMs as they drain.  Captured into CUDA graphs as programmatic edges.
-inline bool pdl_enabled() {
-  static const int v = [] { const char* e = getenv("THMR_PDL"); return e ? atoi(e) : 0; }();
-  return v != 0;
-}
 #ifdef __CUDACC__
 // In-graph timing: the first thread of block 0 of a kernel records the global nanosecond timer at kernel start
 // (nullptr = off).  Kernels of a stream run back to back, so start(next) - start(this) is this kernel's share of the
@@ -121,24 +113,6 @@ __device__ __forceinline__ void stamp_start(unsigned long long* stamp) {
   }
 }
 __global__ void stamp_kernel(unsigned long long* stamp) { stamp_start(stamp); }
-
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
 #endif
 
 inline int num_sms() {

@@ -1,8 +1,6 @@
 // HBM-bound row kernels: patch im2col, LayerNorm, softmax, gathers.  Warp-shuffle reductions, fp32 math,
 // vectorised coalesced loads; outputs are written in the operand format of the consuming tcgen05 GEMM (fp16).
 #pragma once
-#include <stdlib.h>
-
 #include "common.cuh"
 #include "ptx.cuh"
 
@@ -58,8 +56,8 @@ __global__ void im2col_patch_kernel(const float* __restrict__ img, __half* __res
 // ------------------------------------------------------------------------------------------------
 // PLAIN16: the ViT's case (fp16 output only, no ReLU, not transposed, C == 128 * VEC4 exactly), compiled without the other
 // output modes' branches and without the per-chunk column guards.
-template <int VEC4, bool PREFETCH, bool PLAIN16 = false>  // float4 loads per lane; PREFETCH: the next row's loads are issued before this row's math
-__global__ void __launch_bounds__(256, VEC4 > 10 ? (PREFETCH ? 1 : 2) : (PREFETCH ? 2 : 4))
+template <int VEC4, bool PLAIN16 = false>  // float4 loads per lane
+__global__ void __launch_bounds__(256, VEC4 > 10 ? 2 : 4)
 layernorm_reg_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
                      __half* __restrict__ y16, int ld16, float* __restrict__ y32_, int R, int C_, float eps, int relu_,
                      int out_t_, unsigned long long* stamp) {
@@ -73,13 +71,11 @@ layernorm_reg_kernel(const float* __restrict__ x, const float* __restrict__ gamm
   extern __shared__ float4 s_gb[];   // [2][C/4]
   float4* sg = s_gb;
   float4* sb = s_gb + C / 4;
-  pdl_launch_dependents();
   for (int c = threadIdx.x; c < C / 4; c += blockDim.x) {
     sg[c] = reinterpret_cast<const float4*>(gamma)[c];
     sb[c] = reinterpret_cast<const float4*>(beta)[c];
   }
   __syncthreads();
-  pdl_wait();       // gamma / beta are weights; x is the predecessor's output
   const int lane = threadIdx.x & 31;
   const int warps_total = (gridDim.x * blockDim.x) >> 5;
   auto load_row = [&](float4 (&v)[VEC4], int row) {
@@ -91,16 +87,9 @@ layernorm_reg_kernel(const float* __restrict__ x, const float* __restrict__ gamm
     }
   };
   // persistent warps: the grid is sized to the resident capacity and every warp walks rows with a grid stride
-  int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  float4 v[VEC4];
-  if (PREFETCH && warp < R) load_row(v, warp);
-  for (; warp < R; warp += warps_total) {
-    float4 nx[VEC4];
-    if (PREFETCH) {
-      if (warp + warps_total < R) load_row(nx, warp + warps_total);
-    } else {
-      load_row(v, warp);
-    }
+  for (int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; warp < R; warp += warps_total) {
+    float4 v[VEC4];
+    load_row(v, warp);
     // Packed fp32 (FFMA2: two IEEE lanes per instruction) for the three arithmetic passes: the kernel issues ~320
     // instructions per lane and row and sits at 60 % issue utilisation next to its HBM stalls (ncu); packing takes it to ~200.
     // Rows shorter than the register tile hold zeros beyond C (they add 0 to the sum; the variance pass masks them).
@@ -172,10 +161,6 @@ layernorm_reg_kernel(const float* __restrict__ x, const float* __restrict__ gamm
         }
       }
     }
-    if (PREFETCH) {
-#pragma unroll
-      for (int i = 0; i < VEC4; ++i) v[i] = nx[i];
-    }
   }
 }
 
@@ -223,48 +208,27 @@ inline int layernorm_launch(const float* x, const float* gamma, const float* bet
   THMR_CHECK(C % 4 == 0, "layernorm: C=%d not a multiple of 4", C);
   if (ld16 == 0) ld16 = C;
   if (C <= 2048) {
-    static const int prefetch = [] { const char* e = getenv("THMR_LN_PREFETCH"); return e ? atoi(e) : 0; }();
-    static const int env_shape = [] { const char* e = getenv("THMR_LN_SHAPE"); return e ? atoi(e) : 0; }();
-    // Persistent warps walk the rows with a grid stride, so the launch shape decides how evenly the rows divide: 12288 rows
-    // on the 4736 warps of 148 x 4 blocks of 256 threads take 3 rounds with the last one 59 % full; 148 x 7 blocks of 128
-    // threads = 4144 warps take 3 full rounds.  THMR_LN_SHAPE=1 picks, among fully resident shapes, the one with the fewest
-    // idle warp-rounds.  Measured inside the graph (start stamps): 20.3 / 19.9 us per launch (LN1 / LN2) against 19.3 / 18.9 us
-    // for the fixed 256 x 4 shape -- the kernel is not tail-bound (and LN1 = LN2: not an L2-residency effect either), so the
-    // fixed shape stays the default.
-    int threads = 256, bps = prefetch ? 2 : 4;
-    if (env_shape && !prefetch) {
-      double best = -1.0;
-      const int cand[8][2] = {{256, 4}, {256, 3}, {128, 8}, {128, 7}, {128, 6}, {128, 5}, {256, 2}, {128, 4}};
-      for (const auto& cnd : cand) {
-        const long W = static_cast<long>(num_sms()) * cnd[1] * (cnd[0] / 32);
-        const long rounds = (R + W - 1) / W;
-        // efficiency of the last round, discounted a little for low occupancy (latency hiding)
-        const double eff = static_cast<double>(R) / (rounds * W) * (W >= 24L * num_sms() ? 1.0 : 0.97);
-        if (eff > best + 1e-3) { best = eff; threads = cnd[0]; bps = cnd[1]; }
-      }
-    }
+    // Persistent warps walk the rows with a grid stride over 4 resident blocks of 256 threads per SM.  (Launch shapes that
+    // divide the rows more evenly were measured and are not faster: the kernel is not tail-bound.)
+    constexpr int threads = 256;
     const int rows_per_block = threads / 32;
     int grid = (R + rows_per_block - 1) / rows_per_block;
-    const int resident = num_sms() * bps;
+    const int resident = num_sms() * 4;
     if (grid > resident) grid = resident;
-    THMR_CHECK(C % 4 == 0, "layernorm: C must be a multiple of 4");
     const size_t smem = 2 * static_cast<size_t>(C) * sizeof(float);
     const int vec4 = (C / 4 + 31) / 32;
-    const bool plain16 = y16 && !y32 && !relu && out_t == 0 && C == 128 * vec4 && !prefetch;
-#define THMR_LN_LAUNCH(V)                                                                                           \
-  do {                                                                                                             \
-    if (prefetch) THMR_CUDA(launch_pdl(layernorm_reg_kernel<V, true>, grid, threads, smem, st, x, gamma, beta, y16, \
-                                       ld16, y32, R, C, eps, relu, out_t, stamp));                                 \
-    else if (plain16 && V == vec4) THMR_CUDA(launch_pdl(layernorm_reg_kernel<V, false, true>, grid, threads, smem,  \
-                                       st, x, gamma, beta, y16, ld16, y32, R, C, eps, relu, out_t, stamp));        \
-    else THMR_CUDA(launch_pdl(layernorm_reg_kernel<V, false>, grid, threads, smem, st, x, gamma, beta, y16, ld16,   \
-                              y32, R, C, eps, relu, out_t, stamp));                                                \
-  } while (0)
-    if (vec4 <= 1) THMR_LN_LAUNCH(1);
-    else if (vec4 <= 8) THMR_LN_LAUNCH(8);
-    else if (vec4 <= 10) THMR_LN_LAUNCH(10);
-    else THMR_LN_LAUNCH(16);
-#undef THMR_LN_LAUNCH
+    // register tile of 1, 8, 10 or 16 float4 per lane; [1] = the PLAIN16 form, for rows that fill the tile exactly
+    using LnKernel = void (*)(const float*, const float*, const float*, __half*, int, float*, int, int, float, int, int,
+                              unsigned long long*);
+    const int tile[4] = {1, 8, 10, 16};
+    const LnKernel kernels[4][2] = {{layernorm_reg_kernel<1>, layernorm_reg_kernel<1, true>},
+                                    {layernorm_reg_kernel<8>, layernorm_reg_kernel<8, true>},
+                                    {layernorm_reg_kernel<10>, layernorm_reg_kernel<10, true>},
+                                    {layernorm_reg_kernel<16>, layernorm_reg_kernel<16, true>}};
+    const int ti = vec4 <= 1 ? 0 : vec4 <= 8 ? 1 : vec4 <= 10 ? 2 : 3;
+    const bool plain16 = y16 && !y32 && !relu && out_t == 0 && C == 128 * vec4 && vec4 == tile[ti];
+    kernels[ti][plain16 ? 1 : 0]<<<grid, threads, smem, st>>>(x, gamma, beta, y16, ld16, y32, R, C, eps, relu, out_t,
+                                                               stamp);
   } else {
     THMR_CHECK(out_t == 0, "layernorm: transposed output needs C <= 2048");
     layernorm_wide_kernel<<<R, 256, 0, st>>>(x, gamma, beta, y16, ld16, y32, R, C, eps, relu, stamp);

@@ -234,9 +234,6 @@ inline size_t engine_build(thmr_engine* e, void* workspace, int B, bool build, i
     d.bias = bias; d.act = act; d.resid = resid; d.ldr = N;
     d.out32 = o32; d.ld32 = N; d.out16 = o16; d.ld16 = N;
     if (!c.concurrent && gemm_sk_flag_count(rows, N) <= n_skf) d.sk_flags = skf;   // (stream-K spins across CTA pairs)
-    d.a_dead = (A == xn || A == ao || A == hbuf || (A >= xn && A < xn + static_cast<size_t>(M) * D) ||
-                (A >= ao && A < ao + static_cast<size_t>(M) * D) ||
-                (A >= hbuf && A < hbuf + static_cast<size_t>(M) * c.vit_mlp_ratio * D)) ? 1 : 0;
     add_gemm(d);
   };
   auto ln = [&](const float* in, const float* g, const float* b, __half* o16, float* o32, int R, int C, float eps,
@@ -270,45 +267,29 @@ inline size_t engine_build(thmr_engine* e, void* workspace, int B, bool build, i
     d.out32 = x; d.ld32 = D;
     add_gemm(d);
   }
-  // THMR_VIT_SUB=n: run the 32 blocks over sub-batches of n images (all blocks of one sub-batch, then the next), so
-  // that a sub-batch's activations (x, xn, qkv, ao, h: 2.7 MB per image) stay resident in the 126 MB L2 between the
-  // kernel that writes them and the one that reads them; the price is smaller GEMMs (fewer tiles per wave) and the
-  // weights being streamed once per sub-batch.  0 (default) = the whole batch at once.
-  static const int env_sub = [] { const char* v = getenv("THMR_VIT_SUB"); return v ? atoi(v) : 0; }();
-  const int sub = (env_sub > 0 && env_sub < B) ? env_sub : B;
-  for (int b0 = 0; b0 < B; b0 += sub) {
-  const int bn = (B - b0) < sub ? (B - b0) : sub;
-  const int Ms = bn * T;
-  const size_t r0 = static_cast<size_t>(b0) * T;
-  float* xs = x + r0 * D;
-  __half* xns = xn + r0 * D;
-  __half* qkvs = qkv + r0 * 3 * D;
-  __half* aos = ao + r0 * D;
-  __half* hs = hbuf + r0 * c.vit_mlp_ratio * D;
   for (int i = 0; i < c.vit_depth; ++i) {
     const thmr_vit_block& bw = e->blocks[i];
     S.tag("vit.layernorm");
-    ln(xs, bw.ln1_g, bw.ln1_b, xns, nullptr, Ms, D, c.vit_ln_eps, 0, 0);
+    ln(x, bw.ln1_g, bw.ln1_b, xn, nullptr, M, D, c.vit_ln_eps, 0, 0);
     S.tag("vit.qkv_gemm");
-    linear(xns, D, Ms, bw.qkv_w, 3 * D, D, bw.qkv_b, kActNone, nullptr, qkvs);
+    linear(xn, D, M, bw.qkv_w, 3 * D, D, bw.qkv_b, kActNone, nullptr, qkv);
     {
       // 4*N*N*d FLOPs per head (QK^T + PV); Q,K,V read + O written once in fp16
-      S.tag("vit.attention", 4.0 * bn * H * 192.0 * 192.0 * 80.0, 4.0 * Ms * D * 2);
+      S.tag("vit.attention", 4.0 * B * H * 192.0 * 192.0 * 80.0, 4.0 * M * D * 2);
       AttnPlan ap;
-      const int s = attention_make_plan(qkvs, 3 * D, bn, H, aos, D, nullptr, &ap);
+      const int s = attention_make_plan(qkv, 3 * D, B, H, ao, D, nullptr, &ap);
       if (s != THMR_OK) err = s;
       ap.p.stamp = slot();
       S.push_back([ap](const RunCtx&, cudaStream_t st) -> int { return attention_dispatch(ap, st); });
     }
     S.tag("vit.proj_gemm");
-    linear(aos, D, Ms, bw.proj_w, D, D, bw.proj_b, kActNone, xs, nullptr, xs);
+    linear(ao, D, M, bw.proj_w, D, D, bw.proj_b, kActNone, x, nullptr, x);
     S.tag("vit.layernorm");
-    ln(xs, bw.ln2_g, bw.ln2_b, xns, nullptr, Ms, D, c.vit_ln_eps, 0, 0);
+    ln(x, bw.ln2_g, bw.ln2_b, xn, nullptr, M, D, c.vit_ln_eps, 0, 0);
     S.tag("vit.fc1_gelu_gemm");
-    linear(xns, D, Ms, bw.fc1_w, c.vit_mlp_ratio * D, D, bw.fc1_b, kActGelu, nullptr, hs);
+    linear(xn, D, M, bw.fc1_w, c.vit_mlp_ratio * D, D, bw.fc1_b, kActGelu, nullptr, hbuf);
     S.tag("vit.fc2_gemm");
-    linear(hs, c.vit_mlp_ratio * D, Ms, bw.fc2_w, D, c.vit_mlp_ratio * D, bw.fc2_b, kActNone, xs, nullptr, xs);
-  }
+    linear(hbuf, c.vit_mlp_ratio * D, M, bw.fc2_w, D, c.vit_mlp_ratio * D, bw.fc2_b, kActNone, x, nullptr, x);
   }
   {
     S.tag("vit.layernorm", 0, static_cast<double>(M) * D * 6);

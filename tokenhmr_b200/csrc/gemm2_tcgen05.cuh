@@ -11,8 +11,9 @@
 //               "smem slot free" and "accumulator ready" barriers of both CTAs
 //   peer      : its epilogue warps release the accumulator buffer by arriving on the leader's barrier
 //
-// Only the TMA epilogues are supported here (fp16 store, fp32 reduce-add); everything else runs on the
-// single-CTA kernel.  The reduce-add flavour supports split-K (partial tiles add into the output in L2).
+// Only the TMA epilogues are supported here (fp16 store, fp32 store, fp32 reduce-add); everything else runs on the
+// single-CTA kernel.  The reduce-add flavour supports stream-K (partial tiles add into the output in L2, in a fixed
+// order).
 #pragma once
 #include "gemm_tcgen05.cuh"
 
@@ -30,7 +31,7 @@ constexpr uint32_t kG2SmemTotal = kG2BiasOffset + 1024 + 1024;
 static_assert(kG2SmemTotal <= 232448, "CTA-pair GEMM shared memory exceeds 227 KB");
 
 // Work decomposition shared by the three warp roles of a cluster (all of them walk the same item sequence).
-//   classic : tiles (x ksplit) round-robin over the clusters, column tile fastest (clusters running side by side share
+//   classic : whole tiles round-robin over the clusters, column tile fastest (clusters running side by side share
 //             A row blocks and weight column blocks in L2).
 //   stream-K: whole tiles quantise badly when tiles / clusters is small -- proj / fc2 have 240 tiles on 74 clusters, i.e.
 //             3.24 waves rounded up to 4.  Hybrid schedule: the first floor(tiles / clusters) - 1 rounds run classic
@@ -44,15 +45,14 @@ static_assert(kG2SmemTotal <= 232448, "CTA-pair GEMM shared memory exceeds 227 K
 //             blocks at any time, A is re-read from HBM once per column tile, fc2 159 us vs 139 us classic.)
 struct G2Work {
   int tiles_m, tiles_n, num_kb;
-  int tile, dp_tiles, stride, ksplit, kb_per;    // classic phase: flat (tile, k-split) index, < dp_tiles * ksplit
+  int tile, dp_tiles, stride;                    // classic phase: tile index, < dp_tiles
   int u, u_end;                                  // stream-K phase: units (k-blocks) of tiles [dp_tiles, tiles) of this cluster
   int cur_tile, cur_m, cur_n, cur_kb0, cur_kb1;  // the current item
   __device__ void load() {
-    if (tile < dp_tiles * ksplit) {
-      cur_tile = tile / ksplit;
-      const int ks = tile - cur_tile * ksplit;
-      cur_kb0 = ks * kb_per;
-      cur_kb1 = (cur_kb0 + kb_per < num_kb) ? cur_kb0 + kb_per : num_kb;
+    if (tile < dp_tiles) {
+      cur_tile = tile;
+      cur_kb0 = 0;
+      cur_kb1 = num_kb;
     } else {
       const int t = u / num_kb;
       cur_tile = dp_tiles + t;
@@ -65,9 +65,9 @@ struct G2Work {
   }
   // sk_tiles = number of trailing tiles scheduled stream-K (0 = all classic); the host guarantees sk_tiles >= nclusters
   // and sk_tiles * num_kb * nclusters < 2^31
-  __device__ G2Work(int sk_tiles, int tm, int tn, int nkb, int ks, int cluster, int nclusters)
-      : tiles_m(tm), tiles_n(tn), num_kb(nkb), tile(cluster), dp_tiles(tm * tn - sk_tiles), stride(nclusters), ksplit(ks),
-        kb_per((nkb + ks - 1) / ks), u(0), u_end(0) {
+  __device__ G2Work(int sk_tiles, int tm, int tn, int nkb, int cluster, int nclusters)
+      : tiles_m(tm), tiles_n(tn), num_kb(nkb), tile(cluster), dp_tiles(tm * tn - sk_tiles), stride(nclusters), u(0),
+        u_end(0) {
     if (sk_tiles > 0) {
       const long long total = static_cast<long long>(sk_tiles) * nkb;
       u = static_cast<int>(total * cluster / nclusters);
@@ -75,13 +75,13 @@ struct G2Work {
     }
     load();
   }
-  __device__ bool valid() const { return tile < dp_tiles * ksplit || u < u_end; }
+  __device__ bool valid() const { return tile < dp_tiles || u < u_end; }
   __device__ void next() {
-    if (tile < dp_tiles * ksplit) tile += stride;
+    if (tile < dp_tiles) tile += stride;
     else u = (cur_tile - dp_tiles) * num_kb + cur_kb1;
     load();
   }
-  __device__ bool in_streamk() const { return tile >= dp_tiles * ksplit; }
+  __device__ bool in_streamk() const { return tile >= dp_tiles; }
   __device__ int tile_index() const { return cur_tile; }
   __device__ int m_blk() const { return cur_m; }
   __device__ int n_blk() const { return cur_n; }
@@ -92,7 +92,7 @@ struct G2Work {
 template <int EPI>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGemmThreads, 1)
 gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
-                        const __grid_constant__ CUtensorMap tmC, const GemmParams p, const int ksplit) {
+                        const __grid_constant__ CUtensorMap tmC, const GemmParams p) {
   static_assert(EPI == kEpiStore16 || EPI == kEpiAdd32 || EPI == kEpiStore32, "CTA-pair GEMM supports the TMA epilogues only");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -113,7 +113,6 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
   const int num_kb = (p.K + kGemmBK - 1) / kGemmBK;
   const int sk_tiles = (EPI == kEpiAdd32 && p.sk_flags != nullptr) ? p.sk_tiles : 0;
 
-  pdl_launch_dependents();
   stamp_start(p.stamp);
   if (warp == kWarpTma && lane == 0) {
     tma_prefetch_desc(&tmA);
@@ -140,44 +139,26 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
   cluster_sync_all();     // peer barriers initialised, both TMEM allocations done
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  pdl_wait();       // barriers, TMEM and descriptors are set up; operands / outputs belong to the predecessor until here
 
   if (warp == kWarpTma) {
     if (lane == 0) {
       // ------------------------------------------------------------ TMA producer (both CTAs)
       int stage = 0;
       uint32_t phase = 0;
-      long long w_empty = 0;
-      const long long t_begin = clock64();
-      const bool a_hint = (p.l2_hints & 1) != 0;
-      const uint64_t pol_a = l2_policy_evict_first();
-      for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, ksplit, cluster_id, num_clusters); w.valid(); w.next()) {
+      for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, cluster_id, num_clusters); w.valid(); w.next()) {
         const int m0 = w.m_blk() * 2 * kGemmBM + static_cast<int>(rank) * kGemmBM;
         const int n0 = w.n_blk() * kG2BN + static_cast<int>(rank) * (kG2BN / 2);
         const int kb0 = w.kb0();
         const int kb1 = w.kb1();
-        if (EPI == kEpiAdd32 && (p.dbg & 512)) {
-          // experiment (off by default): L2-prefetch this CTA's 128 x 256 fp32 reduce-add target a main loop ahead.
-          // Measured in the step: 18.18 vs 18.01 ms without -- the extra HBM reads arrive while the operands stream.
-#pragma unroll
-          for (int c = 0; c < kG2BN / 32; ++c) tma_prefetch_2d(&tmC, w.n_blk() * kG2BN + c * 32, m0);
-        }
         for (int kb = kb0; kb < kb1; ++kb) {
-          const long long t0 = clock64();
           mbar_wait(&empty_bar[stage], phase ^ 1);
-          w_empty += clock64() - t0;
           uint8_t* sa = smem + stage * kG2StageBytes;
           uint8_t* sb = sa + kG2ABytes;
           if (rank == 0) mbar_arrive_expect_tx(&full_bar[stage], 2 * kG2StageBytes);
-          if (a_hint) tma_load_2d_2sm_hint(sa, &tmA, &full_bar[stage], kb * kGemmBK, m0, pol_a);
-          else tma_load_2d_2sm(sa, &tmA, &full_bar[stage], kb * kGemmBK, m0);
+          tma_load_2d_2sm(sa, &tmA, &full_bar[stage], kb * kGemmBK, m0);
           tma_load_2d_2sm(sb, &tmB, &full_bar[stage], kb * kGemmBK, n0);
           if (++stage == kG2Stages) { stage = 0; phase ^= 1; }
         }
-      }
-      if (p.dbg_counters) {
-        p.dbg_counters[blockIdx.x * 16 + 0] = w_empty;
-        p.dbg_counters[blockIdx.x * 16 + 1] = clock64() - t_begin;
       }
     }
   } else if (warp == kWarpMma) {
@@ -197,23 +178,15 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      long long w_tempty = 0, w_full = 0;
-      const long long t_begin = clock64();
       bool ready = false;
-      for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, ksplit, cluster_id, num_clusters); w.valid(); w.next()) {
+      for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, cluster_id, num_clusters); w.valid(); w.next()) {
         const int kb0 = w.kb0();
         const int kb1 = w.kb1();
-        long long t0 = clock64();
         mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        w_tempty += clock64() - t0;
         tc_fence_after();
         const uint32_t d_tmem = tmem_u + acc * kG2BN;
         for (int kb = kb0; kb < kb1; ++kb) {
-          if (!ready) {
-            t0 = clock64();
-            mbar_wait(&full_bar[stage], phase);
-            w_full += clock64() - t0;
-          }
+          if (!ready) mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
           const uint32_t sa = smem_base + stage * kG2StageBytes;
           const uint32_t sb = sa + kG2ABytes;
@@ -236,11 +209,6 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
         }
         if ((acc ^= 1) == 0) acc_phase ^= 1;
       }
-      if (p.dbg_counters && lane == 0) {
-        p.dbg_counters[blockIdx.x * 16 + 2] = w_tempty;
-        p.dbg_counters[blockIdx.x * 16 + 3] = w_full;
-        p.dbg_counters[blockIdx.x * 16 + 4] = clock64() - t_begin;
-      }
     }
   } else if (warp < kGemmEpiWarps) {
     // -------------------------------------------------------------- epilogue (both CTAs, own 128 rows)
@@ -252,20 +220,18 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
     uint8_t* stage_buf = smem + kG2StagingOffset + warp * 4096;
     // Slab stores: the four row-quarter warps of a column half stage their 32 rows side by side (their 4 KB buffers are
     // contiguous and share the 128B-swizzle phase), meet at a named barrier and ONE thread issues a 128-row TMA store:
-    // 4 (fp16) / 8 (fp32) TMA operations per tile and CTA instead of 16 / 32.  THMR_GEMM_DBG bit 7 = per-warp stores.
-    const bool slab = !(p.dbg & 128);
+    // 4 (fp16) / 8 (fp32) TMA operations per tile and CTA instead of 16 / 32.
     uint8_t* slab_buf = smem + kG2StagingOffset + half * 4 * 4096;
-    // Bias of the tile's column half in shared memory (slab mode): each of the half's four warps writes the same 128
+    // Bias of the tile's column half in shared memory (fp16 epilogue): each of the half's four warps writes the same 128
     // values and reads them back as broadcast 16-byte loads -- one LDS per 4 columns instead of 4 shuffles.  The named
     // barriers of the slab stores keep the four warps inside the same tile, so one buffer per half is enough: nobody
     // reads the previous tile's bias after the last chunk's barrier.
     float* sbias = reinterpret_cast<float*>(smem + kG2BiasOffset) + half * 128;
-    const bool packed = slab && !(p.dbg & 256);     // THMR_GEMM_DBG bit 8: the scalar / shuffle epilogue (A/B)
     const uint32_t srow = smem_u32(stage_buf) + lane * 128;
     const int sw = lane & 7;
     int acc = 0;
     uint32_t acc_phase = 0;
-    for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, ksplit, cluster_id, num_clusters); w.valid(); w.next()) {
+    for (G2Work w(sk_tiles, tiles_m, tiles_n, num_kb, cluster_id, num_clusters); w.valid(); w.next()) {
       const int m0 = w.m_blk() * 2 * kGemmBM + static_cast<int>(rank) * kGemmBM;
       const int n0 = w.n_blk() * kG2BN;
       const bool add_bias = p.bias && w.kb0() == 0;
@@ -283,7 +249,7 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
         const int bc = n0 + half * (kG2BN / 2) + lane * 4;
         if (add_bias && lane * 4 < kG2BN / 2 && bc < p.N) bq = __ldg(reinterpret_cast<const float4*>(p.bias + bc));
       }
-      if (packed) {
+      if constexpr (EPI == kEpiStore16) {
         *reinterpret_cast<float4*>(sbias + lane * 4) = bq;
         __syncwarp();
       }
@@ -291,73 +257,41 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
       __syncwarp();
       tc_fence_after();
 #pragma unroll 1
-      for (int cc = 0; cc < ((p.dbg & 1) ? 0 : kChunksPerHalf); ++cc) {
+      for (int cc = 0; cc < kChunksPerHalf; ++cc) {
         const int c = half * kChunksPerHalf + cc;
         const int col0 = n0 + c * kChunkCols;
         uint32_t pk[32];
         if constexpr (EPI == kEpiStore16) {
-          if (packed) {
-            // packed fp32 path: bias add, GELU and the fp16 conversion two columns at a time
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-              uint32_t v[32];
-              tmem_ld_x32(tmem_base + lane_addr + acc * kG2BN + c * 64 + hh * 32, v);
-              tmem_ld_wait();
-              uint64_t f2[16];
-#pragma unroll
-              for (int j = 0; j < 32; j += 4) {
-                const float4 b4 = *reinterpret_cast<const float4*>(sbias + cc * 64 + hh * 32 + j);   // broadcast
-                f2[j >> 1] = f2_add(f2_pack(__uint_as_float(v[j]), __uint_as_float(v[j + 1])), f2_pack(b4.x, b4.y));
-                f2[(j >> 1) + 1] = f2_add(f2_pack(__uint_as_float(v[j + 2]), __uint_as_float(v[j + 3])), f2_pack(b4.z, b4.w));
-              }
-              if (p.act == kActGelu) {
-#pragma unroll
-                for (int j = 0; j < 16; ++j) f2[j] = gelu_erf2(f2[j]);
-              } else if (p.act == kActRelu) {
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                  float a, b;
-                  f2_unpack(f2[j], a, b);
-                  f2[j] = f2_pack(fmaxf(a, 0.f), fmaxf(b, 0.f));
-                }
-              }
-#pragma unroll
-              for (int j = 0; j < 16; ++j) {
-                float a, b;
-                f2_unpack(f2[j], a, b);
-                __half2 h2 = __floats2half2_rn(a, b);
-                pk[hh * 16 + j] = *reinterpret_cast<uint32_t*>(&h2);
-              }
-            }
-          } else
+          // packed fp32 path: bias add, GELU and the fp16 conversion two columns at a time
 #pragma unroll
           for (int hh = 0; hh < 2; ++hh) {
             uint32_t v[32];
             tmem_ld_x32(tmem_base + lane_addr + acc * kG2BN + c * 64 + hh * 32, v);
             tmem_ld_wait();
-            float f[32];
+            uint64_t f2[16];
 #pragma unroll
             for (int j = 0; j < 32; j += 4) {
-              const int bl = (cc * 64 + hh * 32 + j) >> 2;   // lane holding these 4 columns' bias
-              float4 b4;
-              b4.x = __shfl_sync(0xffffffffu, bq.x, bl); b4.y = __shfl_sync(0xffffffffu, bq.y, bl);
-              b4.z = __shfl_sync(0xffffffffu, bq.z, bl); b4.w = __shfl_sync(0xffffffffu, bq.w, bl);
-              f[j] = __uint_as_float(v[j]) + b4.x; f[j + 1] = __uint_as_float(v[j + 1]) + b4.y;
-              f[j + 2] = __uint_as_float(v[j + 2]) + b4.z; f[j + 3] = __uint_as_float(v[j + 3]) + b4.w;
+              const float4 b4 = *reinterpret_cast<const float4*>(sbias + cc * 64 + hh * 32 + j);   // broadcast
+              f2[j >> 1] = f2_add(f2_pack(__uint_as_float(v[j]), __uint_as_float(v[j + 1])), f2_pack(b4.x, b4.y));
+              f2[(j >> 1) + 1] = f2_add(f2_pack(__uint_as_float(v[j + 2]), __uint_as_float(v[j + 3])), f2_pack(b4.z, b4.w));
             }
-            // warp-uniform branch OUTSIDE the element loop (otherwise the compiler if-converts it and every element
-            // pays for GELU and ReLU even when no activation is requested)
             if (p.act == kActGelu) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) f[j] = gelu_erf(f[j]);
+              for (int j = 0; j < 16; ++j) f2[j] = gelu_erf2(f2[j]);
             } else if (p.act == kActRelu) {
 #pragma unroll
-              for (int j = 0; j < 32; ++j) f[j] = fmaxf(f[j], 0.f);
+              for (int j = 0; j < 16; ++j) {
+                float a, b;
+                f2_unpack(f2[j], a, b);
+                f2[j] = f2_pack(fmaxf(a, 0.f), fmaxf(b, 0.f));
+              }
             }
 #pragma unroll
-            for (int j = 0; j < 32; j += 2) {
-              __half2 h2 = __floats2half2_rn(f[j], f[j + 1]);
-              pk[hh * 16 + (j >> 1)] = *reinterpret_cast<uint32_t*>(&h2);
+            for (int j = 0; j < 16; ++j) {
+              float a, b;
+              f2_unpack(f2[j], a, b);
+              __half2 h2 = __floats2half2_rn(a, b);
+              pk[hh * 16 + j] = *reinterpret_cast<uint32_t*>(&h2);
             }
           }
         } else {
@@ -376,13 +310,8 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
             pk[j + 3] = __float_as_uint(fmaf(p.alpha, __uint_as_float(v[j + 3]), b4.w));
           }
         }
-        if (slab) {
-          if (q == 0 && lane == 0) tma_store_wait_read<0>();     // the previous slab has been read out of smem
-          named_bar_sync_128(1 + half);
-        } else {
-          if (lane == 0) tma_store_wait_read<0>();
-          __syncwarp();
-        }
+        if (q == 0 && lane == 0) tma_store_wait_read<0>();     // the previous slab has been read out of smem
+        named_bar_sync_128(1 + half);
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(srow + ((j ^ sw) << 4)), "r"(pk[4 * j]),
@@ -390,40 +319,29 @@ gemm_f16_tn_2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                        : "memory");
         }
         fence_proxy_async_smem();
-        if (slab) {
-          named_bar_sync_128(1 + half);
-          if (q == 0 && lane == 0 && col0 < p.N && m0 < p.M && !(p.dbg & 2)) {
-            if constexpr (EPI == kEpiStore16) tma_store_2d(&tmC, slab_buf, col0, m0);
-            else if constexpr (EPI == kEpiStore32) tma_store_2d(&tmC, slab_buf, col0, m0);
-            else {
-              if (sk_head && !sk_waited) {
-                uint32_t it = 0;
-                while (ld_acquire_gpu(sk_flag) == 0u && ++it < kSpinLimit) {}
-                if (it >= kSpinLimit) atomicExch(&g_pipeline_timeout, 1u);
-                *sk_flag = 0u;                      // consumed: ready for the next launch
-                fence_proxy_async_all();
-                sk_waited = true;
-              }
-              if (p.l2_hints & 4) tma_reduce_add_2d_hint(&tmC, slab_buf, col0, m0, l2_policy_evict_last());
-              else tma_reduce_add_2d(&tmC, slab_buf, col0, m0);
+        named_bar_sync_128(1 + half);
+        if (q == 0 && lane == 0 && col0 < p.N && m0 < p.M) {
+          if constexpr (EPI == kEpiStore16) tma_store_2d(&tmC, slab_buf, col0, m0);
+          else if constexpr (EPI == kEpiStore32) tma_store_2d(&tmC, slab_buf, col0, m0);
+          else {
+            if (sk_head && !sk_waited) {
+              uint32_t it = 0;
+              while (ld_acquire_gpu(sk_flag) == 0u && ++it < kSpinLimit) {}
+              if (it >= kSpinLimit) atomicExch(&g_pipeline_timeout, 1u);
+              *sk_flag = 0u;                      // consumed: ready for the next launch
+              fence_proxy_async_all();
+              sk_waited = true;
             }
-            tma_store_commit();
+            tma_reduce_add_2d(&tmC, slab_buf, col0, m0);
           }
-        } else {
-          __syncwarp();
-          if (lane == 0 && col0 < p.N && m0 + q * 32 < p.M && !(p.dbg & 2)) {
-            if constexpr (EPI == kEpiStore16) tma_store_2d(&tmC, stage_buf, col0, m0 + q * 32);
-            else if constexpr (EPI == kEpiStore32) tma_store_2d(&tmC, stage_buf, col0, m0 + q * 32);
-            else tma_reduce_add_2d(&tmC, stage_buf, col0, m0 + q * 32);
-            tma_store_commit();
-          }
+          tma_store_commit();
         }
       }
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive_cluster(&tempty_bar[acc], 0);   // accumulator buffer free (leader's barrier)
       if ((acc ^= 1) == 0) acc_phase ^= 1;
-      if (sk_tail && slab && q == 0 && lane == 0) {
+      if (sk_tail && q == 0 && lane == 0) {
         // every reduce-add of this partial tile has been performed in L2: let the head part go
         tma_store_wait<0>();
         fence_proxy_async_all();

@@ -1,7 +1,6 @@
 // Host side of the tcgen05 GEMM: plan construction (TMA descriptors, tile choice) and launch.
 #pragma once
 #include "common.cuh"
-#include <stdlib.h>
 
 #include "gemm2_tcgen05.cuh"
 #include "gemm_tcgen05.cuh"
@@ -15,7 +14,6 @@ struct GemmPlan {
   int epi;
   int grid;
   int two_cta;  // CTA-pair kernel (256 x 256 tiles)
-  int ksplit;   // split-K factor (reduce-add epilogue only)
 };
 
 struct GemmDesc {
@@ -40,7 +38,6 @@ struct GemmDesc {
   int force_epi = -1;  // 0 forces the generic epilogue (tests)
   int force_2cta = -1; // -1 auto, 0 never, 1 always (when eligible)
   unsigned int* sk_flags = nullptr;  // >= gemm_sk_flag_count(M, N) zeroed uints: enables stream-K for reduce-add GEMMs
-  int a_dead = 0;    // the A operand is not read again after this GEMM: load it with the L2 evict_first policy
   unsigned long long* stamp = nullptr;   // in-graph start stamp slot (nullable)
 };
 
@@ -120,8 +117,6 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   p.out32 = d.out32; p.ld32 = d.ld32; p.out16 = d.out16; p.ld16 = d.ld16;
   p.bias = d.bias; p.resid = d.resid; p.ldr = d.ldr; p.resid_mod = d.resid_mod; p.act = d.act; p.act32 = d.act32;
   p.seq_pitch = d.seq_pitch; p.seq_lo = d.seq_lo; p.seq_hi = d.seq_hi;
-  { const char* e = getenv("THMR_GEMM_DBG"); p.dbg = e ? atoi(e) : 0; }
-  { const char* e = getenv("THMR_GEMM_COUNTERS"); p.dbg_counters = e ? reinterpret_cast<unsigned long long*>(strtoull(e, nullptr, 0)) : nullptr; }
   p.alpha = d.alpha; p.argmin_out = d.argmin_out; p.row_sq = d.row_sq; p.col_sq = d.col_sq;
   THMR_CHECK(!d.screen_rows || (d.argmin_out && d.screen_count && d.screen_cmax2 && d.N % 32 == 0),
              "gemm: screened arg-min needs its queue and N %% 32 == 0");
@@ -129,9 +124,6 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   p.screen_rows = d.screen_rows; p.screen_count = d.screen_count; p.screen_cmax2 = d.screen_cmax2;
   p.screen_rel = d.screen_rel; p.screen_abs = d.screen_abs; p.screen_row0 = d.screen_row0;
   p.row_map = d.row_map; p.m_dev = d.m_dev; p.m_dev_off = d.m_dev_off;
-  // THMR_L2_HINTS bits: 1 = dead A operands evict_first, 2 = attention Q/K/V evict_first, 4 = reduce-add target evict_last
-  static const int env_hints = [] { const char* e = getenv("THMR_L2_HINTS"); return e ? atoi(e) : 0; }();
-  p.l2_hints = ((env_hints & 1) && d.a_dead ? 1 : 0) | (env_hints & 4);
   p.stamp = d.stamp;
   const int num_kb = (d.K + kGemmBK - 1) / kGemmBK;
   uint64_t a_cols = d.K;
@@ -143,20 +135,18 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   } else {
     p.kblocks_per_tap = num_kb;
   }
-  // CTA-pair kernel for the large TMA-epilogue GEMMs (the ViT projections): env THMR_GEMM_2CTA=0 disables it
-  static const int env_2cta = [] { const char* e = getenv("THMR_GEMM_2CTA"); return e ? atoi(e) : 1; }();
-  bool two = epi != kEpiGeneric && d.taps == 1 && d.M >= 256 && d.N >= 256 && !d.force_bn && env_2cta != 0;
+  // CTA-pair kernel for the large TMA-epilogue GEMMs (the ViT projections)
+  bool two = epi != kEpiGeneric && d.taps == 1 && d.M >= 256 && d.N >= 256 && !d.force_bn;
   if (d.force_2cta == 0) two = false;
   if (d.force_2cta == 1 || d.force_bn == 512) two = epi != kEpiGeneric && d.taps == 1;
   plan->two_cta = two ? 1 : 0;
-  plan->ksplit = 1;
   THMR_TRY(make_tmap_2d_f16(&plan->tmA, d.A, d.a_rows, a_cols, d.lda, kGemmBM, kGemmBK, CU_TENSOR_MAP_SWIZZLE_128B));
   const int b_box_rows = two ? kG2BN / 2 : bn;
   THMR_TRY(make_tmap_2d_f16(&plan->tmB, d.B, d.N, d.K, d.ldb, b_box_rows, kGemmBK, CU_TENSOR_MAP_SWIZZLE_128B));
   plan->bn = two ? kG2BN : bn;
   plan->epi = epi;
-  // output boxes: 32 rows per epilogue warp, or (CTA-pair kernel, default) one 128-row slab per column half
-  const uint32_t c_rows = (two && !(p.dbg & 128)) ? 128 : 32;
+  // output boxes: 32 rows per epilogue warp, or (CTA-pair kernel) one 128-row slab per column half
+  const uint32_t c_rows = two ? 128 : 32;
   if (epi == kEpiStore16)
     THMR_TRY(make_tmap_2d(&plan->tmC, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, d.out16, d.M, d.N, d.ld16, c_rows, 64,
                           CU_TENSOR_MAP_SWIZZLE_128B));
@@ -168,31 +158,15 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   if (two) {
     const int clusters = num_sms() / 2;
     const long tiles = static_cast<long>((d.M + 255) / 256) * ((d.N + kG2BN - 1) / kG2BN);
-    // Split-K makes two partial tiles reduce-add into the same output element in arbitrary order: faster when
-    // the tile count quantises badly over the 74 CTA pairs (fc2: +5 %), but not bit-reproducible run to run,
-    // so it is opt-in (THMR_GEMM_SPLITK=1).
-    static const int env_splitk = [] { const char* e = getenv("THMR_GEMM_SPLITK"); return e ? atoi(e) : 0; }();
-    if (epi == kEpiAdd32 && env_splitk) {
-      double best_eff = 0;
-      for (int ks = 1; ks <= 4; ks *= 2) {
-        if (ks > 1 && num_kb / ks < 16) break;
-        const long t = tiles * ks;
-        const double eff = static_cast<double>(t) / (((t + clusters - 1) / clusters) * clusters);
-        if (eff > best_eff + 0.05) { best_eff = eff; plan->ksplit = ks; }
-      }
-    }
-    const long t = tiles * plan->ksplit;
-    plan->grid = 2 * static_cast<int>(t < clusters ? t : clusters);
+    plan->grid = 2 * static_cast<int>(tiles < clusters ? tiles : clusters);
     // Stream-K (gemm2_tcgen05.cuh) when whole tiles quantise badly over the clusters: needs the reduce-add epilogue,
-    // caller-provided ordering flags, at least two tiles of work per cluster (a tile is then shared by at most two
-    // clusters) and the slab stores (their issuing threads own the flags).  THMR_GEMM_STREAMK=0 disables it.
-    static const int env_sk = [] { const char* e = getenv("THMR_GEMM_STREAMK"); return e ? atoi(e) : 1; }();
+    // caller-provided ordering flags and at least two tiles of work per cluster (a tile is then shared by at most two
+    // clusters).
     p.sk_flags = nullptr;
     p.sk_tiles = 0;
     // Short tiles do not pay: every partial tile costs a full 128 x 256 fp32 epilogue, which a 10-k-block main loop no
     // longer hides (proj, 20 k-blocks per tile: 45.3 us with stream-K vs 42.5 us without; fc2, 80: 126.7 vs 138.8 us).
-    if (epi == kEpiAdd32 && d.sk_flags && env_sk && plan->ksplit == 1 && !(p.dbg & 128) && tiles >= 2L * clusters &&
-        tiles % clusters != 0 && num_kb >= 40) {
+    if (epi == kEpiAdd32 && d.sk_flags && tiles >= 2L * clusters && tiles % clusters != 0 && num_kb >= 40) {
       const double eff = static_cast<double>(tiles) / (((tiles + clusters - 1) / clusters) * clusters);
       const long sk_tiles = tiles % clusters + clusters;      // the last partial round plus one full round
       if (eff < 0.97 && static_cast<double>(sk_tiles) * num_kb * clusters < 2.0e9) {
@@ -205,9 +179,8 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   }
   const long tiles_m = (d.M + kGemmBM - 1) / kGemmBM;
   const long tiles = d.argmin_out ? tiles_m : tiles_m * ((d.N + bn - 1) / bn);
-  // the CTAs of a wave should share tiles of the larger operand (TileIter); THMR_GEMM_MFAST=0 keeps column-fastest order
-  static const int env_mfast = [] { const char* e = getenv("THMR_GEMM_MFAST"); return e ? atoi(e) : 1; }();
-  p.m_fast = (env_mfast && !d.argmin_out && tiles_m > 1 && d.M < d.N) ? 1 : 0;
+  // the CTAs of a wave should share tiles of the larger operand (TileIter)
+  p.m_fast = (!d.argmin_out && tiles_m > 1 && d.M < d.N) ? 1 : 0;
   plan->grid = static_cast<int>(tiles < num_sms() ? tiles : num_sms());
   return THMR_OK;
 }
@@ -235,8 +208,8 @@ inline int gemm2_launch_t(const GemmPlan& plan, cudaStream_t stream) {
                                    kG2SmemTotal));
     configured = true;
   }
-  THMR_CUDA(launch_pdl(gemm_f16_tn_2cta_kernel<EPI>, plan.grid, kGemmThreads, kG2SmemTotal, stream, plan.tmA, plan.tmB,
-                       plan.tmC, plan.p, plan.ksplit));
+  gemm_f16_tn_2cta_kernel<EPI><<<plan.grid, kGemmThreads, kG2SmemTotal, stream>>>(plan.tmA, plan.tmB, plan.tmC, plan.p);
+  THMR_CUDA(cudaGetLastError());
   return THMR_OK;
 }
 

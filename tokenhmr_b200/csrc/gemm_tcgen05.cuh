@@ -71,9 +71,6 @@ struct GemmParams {
   int sk_tiles;   // trailing tiles scheduled stream-K (gemm2_tcgen05.cuh G2Work)
   unsigned long long* stamp;   // in-graph start stamp (common.cuh stamp_start), nullable
   int m_fast;     // 1-CTA kernel: row tile fastest in the tile order (see TileIter)
-  int l2_hints;   // CTA-pair kernel: bit 0 = A operand loaded evict_first (dead after this GEMM), bit 2 = reduce-add evict_last
-  unsigned long long* dbg_counters;  // optional [gridDim.x][8] cycle counters (scripts/dev_gemm_qkv.py)
-  int dbg;                 // THMR_GEMM_DBG experiments: 1 = skip epilogue work, 2 = skip only the TMA store
 };
 
 // Tile order shared by the three warp roles.  Normal mode: tiles round-robin over CTAs, column tile
@@ -171,13 +168,6 @@ __device__ __forceinline__ void named_bar_sync_64(int id) {
 __device__ __forceinline__ void named_bar_sync_128(int id) {
   asm volatile("bar.sync %0, 128;" ::"r"(id) : "memory");
 }
-__device__ __forceinline__ void tma_reduce_add_2d_hint(const CUtensorMap* m, const void* smem_src, int32_t c0, int32_t c1,
-                                                       uint64_t policy) {
-  asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group.L2::cache_hint [%0, {%2, %3}], [%1], %4;"
-               :
-               : "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "l"(policy)
-               : "memory");
-}
 __device__ __forceinline__ void tma_reduce_add_2d(const CUtensorMap* m, const void* smem_src, int32_t c0, int32_t c1) {
   asm volatile("cp.reduce.async.bulk.tensor.2d.global.shared::cta.add.bulk_group [%0, {%2, %3}], [%1];"
                :
@@ -250,15 +240,11 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       // ------------------------------------------------------------ TMA producer
       int stage = 0;
       uint32_t phase = 0;
-      long long w_empty = 0;
-      const long long t_begin = clock64();
       for (TileIter it(tiles_m, tiles_n, p.argmin_out != nullptr, p.m_fast != 0); it.valid(); it.next()) {
         const int m0 = it.m0(kGemmBM);
         const int n0 = it.n0(BN);
         for (int kb = 0; kb < num_kb; ++kb) {
-          const long long t0 = clock64();
           mbar_wait(&empty_bar[stage], phase ^ 1);
-          w_empty += clock64() - t0;
           uint8_t* sa = smem + stage * S::kStageBytes;
           uint8_t* sb = sa + S::kABytes;
           const int tap = kb / p.kblocks_per_tap;
@@ -268,10 +254,6 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           tma_load_2d(sb, &tmB, &full_bar[stage], kb * kGemmBK, n0);
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
-      }
-      if (p.dbg_counters) {
-        p.dbg_counters[blockIdx.x * 16 + 0] = w_empty;
-        p.dbg_counters[blockIdx.x * 16 + 1] = clock64() - t_begin;
       }
     }
   } else if (warp == kWarpMma) {
@@ -286,23 +268,15 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      long long w_tempty = 0, w_full = 0;
-      const long long t_begin = clock64();
       // The readiness of the NEXT smem stage is probed right after the MMA issues of the current one, so the latency of
       // mbarrier.try_wait (~100-200 cycles even when the phase is complete) overlaps with tensor work.
       bool ready = false;
       for (TileIter it(tiles_m, tiles_n, p.argmin_out != nullptr, p.m_fast != 0); it.valid(); it.next()) {
-        long long t0 = clock64();
         mbar_wait(&tempty_bar[acc], acc_phase ^ 1);
-        w_tempty += clock64() - t0;
         tc_fence_after();
         const uint32_t d_tmem = tmem_u + acc * BN;
         for (int kb = 0; kb < num_kb; ++kb) {
-          if (!ready) {
-            t0 = clock64();
-            mbar_wait(&full_bar[stage], phase);
-            w_full += clock64() - t0;
-          }
+          if (!ready) mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
           const uint32_t sa = smem_base + stage * S::kStageBytes;
           const uint32_t sb = sa + S::kABytes;
@@ -324,11 +298,6 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
           phase = nphase;
         }
         if ((acc ^= 1) == 0) acc_phase ^= 1;
-      }
-      if (p.dbg_counters && lane == 0) {
-        p.dbg_counters[blockIdx.x * 16 + 2] = w_tempty;
-        p.dbg_counters[blockIdx.x * 16 + 3] = w_full;
-        p.dbg_counters[blockIdx.x * 16 + 4] = clock64() - t_begin;
       }
     }
   } else if (warp < kGemmEpiWarps) {
@@ -558,8 +527,6 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       uint8_t* stage_buf = smem + S::kStagingOffset + warp * 4096;   // [32 rows][128 B], 128B-swizzled
       const uint32_t srow = smem_u32(stage_buf) + lane * 128;
       const int sw = lane & 7;
-      long long w_tfull = 0, w_store = 0, w_ldtm = 0, w_alu = 0, w_sts = 0, w_fence = 0;
-      const long long t_begin = clock64();
       for (TileIter it(tiles_m, tiles_n, false, p.m_fast != 0); it.valid(); it.next()) {
         const int m0 = it.m0(kGemmBM);
         const int n0 = it.n0(BN);
@@ -567,32 +534,22 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         float4 bq = make_float4(0.f, 0.f, 0.f, 0.f);
         {
           const int bc = n0 + half * (BN / 2) + lane * 4;
-          if (p.bias && !(p.dbg & 8) && lane * 4 < BN / 2 && bc < p.N) bq = __ldg(reinterpret_cast<const float4*>(p.bias + bc));
+          if (p.bias && lane * 4 < BN / 2 && bc < p.N) bq = __ldg(reinterpret_cast<const float4*>(p.bias + bc));
         }
-        const long long t0 = clock64();
         if (lane == 0) mbar_wait(&tfull_bar[acc], acc_phase);   // one polling lane per warp
         __syncwarp();
-        w_tfull += clock64() - t0;
         tc_fence_after();
 #pragma unroll 1
-        const int my_chunks = (p.dbg & 1) ? 0 : kChunksPerHalf;
-        for (int cc = 0; cc < my_chunks; ++cc) {
+        for (int cc = 0; cc < kChunksPerHalf; ++cc) {
           const int c = half * kChunksPerHalf + cc;
           const int col0 = n0 + c * kChunkCols;
           uint32_t pk[32];
-          long long tq = clock64();
           if constexpr (EPI == kEpiStore16) {
 #pragma unroll
             for (int hh = 0; hh < 2; ++hh) {
               uint32_t v[32];
-              if (!(p.dbg & 32)) {
-                tmem_ld_x32(tmem_base + lane_addr + acc * BN + c * 64 + hh * 32, v);
-                tmem_ld_wait();
-                { const long long tn = clock64(); w_ldtm += tn - tq; tq = tn; }
-              } else {
-#pragma unroll
-                for (int j = 0; j < 32; ++j) v[j] = j + lane;
-              }
+              tmem_ld_x32(tmem_base + lane_addr + acc * BN + c * 64 + hh * 32, v);
+              tmem_ld_wait();
               float f[32];
 #pragma unroll
               for (int j = 0; j < 32; j += 4) {
@@ -617,7 +574,6 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
                 __half2 h2 = __floats2half2_rn(f[j], f[j + 1]);
                 pk[hh * 16 + (j >> 1)] = *reinterpret_cast<uint32_t*>(&h2);
               }
-              { const long long tn = clock64(); w_alu += tn - tq; tq = tn; }
             }
           } else {
             uint32_t v[32];
@@ -636,26 +592,17 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
             }
           }
           // the previous TMA store of this warp must have finished reading the staging tile
-          const long long tw0 = clock64();
           if (lane == 0) tma_store_wait_read<0>();
           __syncwarp();
-          w_store += clock64() - tw0;
-          if (!(p.dbg & 16)) {
 #pragma unroll
-            for (int j = 0; j < 8; ++j) {
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(srow + ((j ^ sw) << 4)), "r"(pk[4 * j]),
-                           "r"(pk[4 * j + 1]), "r"(pk[4 * j + 2]), "r"(pk[4 * j + 3])
-                           : "memory");
-            }
-            { const long long tn = clock64(); w_sts += tn - tw0 - 0; }
-            const long long tf0 = clock64();
-            if (!(p.dbg & 64)) fence_proxy_async_smem();
-            w_fence += clock64() - tf0;
-          } else if (pk[0] == 0x12345678u && pk[31] == 0x9abcdef0u) {
-            asm volatile("st.shared.b32 [%0], %1;" ::"r"(srow), "r"(pk[7]) : "memory");
+          for (int j = 0; j < 8; ++j) {
+            asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(srow + ((j ^ sw) << 4)), "r"(pk[4 * j]),
+                         "r"(pk[4 * j + 1]), "r"(pk[4 * j + 2]), "r"(pk[4 * j + 3])
+                         : "memory");
           }
+          fence_proxy_async_smem();
           __syncwarp();
-          if (lane == 0 && col0 < p.N && m0 + q * 32 < M_eff && !(p.dbg & 2)) {
+          if (lane == 0 && col0 < p.N && m0 + q * 32 < M_eff) {
             if constexpr (EPI == kEpiStore16) tma_store_2d(&tmC, stage_buf, col0, m0 + q * 32);
             else if constexpr (EPI == kEpiStore32) tma_store_2d(&tmC, stage_buf, col0, m0 + q * 32);
             else tma_reduce_add_2d(&tmC, stage_buf, col0, m0 + q * 32);
@@ -666,15 +613,6 @@ gemm_f16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         __syncwarp();
         if (lane == 0) mbar_arrive(&tempty_bar[acc]);
         if ((acc ^= 1) == 0) acc_phase ^= 1;
-      }
-      if (p.dbg_counters && warp == 0 && lane == 0) {
-        p.dbg_counters[blockIdx.x * 16 + 5] = w_tfull;
-        p.dbg_counters[blockIdx.x * 16 + 6] = clock64() - t_begin;
-        p.dbg_counters[blockIdx.x * 16 + 7] = w_store;
-        p.dbg_counters[blockIdx.x * 16 + 8] = w_ldtm;
-        p.dbg_counters[blockIdx.x * 16 + 9] = w_alu;
-        p.dbg_counters[blockIdx.x * 16 + 10] = w_sts;
-        p.dbg_counters[blockIdx.x * 16 + 11] = w_fence;
       }
       if (lane == 0) tma_store_wait<0>();   // all bulk stores complete before the CTA exits
     }

@@ -117,28 +117,6 @@ __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m
         "r"(c2)
       : "memory");
 }
-// L2 eviction-priority policies for TMA traffic (createpolicy): evict_first for operands that are dead once this kernel
-// has read them (activations), evict_last for data the next kernel needs (the residual stream).
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void tma_load_3d_hint(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int32_t c0,
-                                                 int32_t c1, int32_t c2, uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4, %5}], [%2], %6;"
-      :
-      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1),
-        "r"(c2), "l"(policy)
-      : "memory");
-}
 // 2D tiled store shared -> global (bulk group completion).
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* smem_src, int32_t c0, int32_t c1) {
   asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
@@ -147,13 +125,6 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* m, const void* s
                : "memory");
 }
 __device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// L2 prefetch of one tensor-map box (no shared-memory destination, no completion to wait for).
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int32_t c0, int32_t c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];"
-               :
-               : "l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-               : "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
 __device__ __forceinline__ uint32_t ld_acquire_gpu(const uint32_t* p) {
   uint32_t v;
@@ -353,16 +324,6 @@ __device__ __forceinline__ void tma_load_2d_2sm(void* smem_dst, const CUtensorMa
       :
       : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0),
         "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_2sm_hint(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int32_t c0,
-                                                     int32_t c1, uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint"
-      " [%0], [%1, {%3, %4}], [%2], %5;"
-      :
-      : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0),
-        "r"(c1), "l"(policy)
       : "memory");
 }
 __device__ __forceinline__ void tmem_alloc_2sm(uint32_t* smem_slot, uint32_t ncols) {
