@@ -319,7 +319,8 @@ size_t thmr_engine_workspace_bytes(const thmr_engine* e, int max_batch);
  * thmr_engine_workspace_bytes(e, B) bytes, 1024-byte aligned. */
 int thmr_engine_forward(thmr_engine* e, const float* img, int B, const thmr_outputs* out, void* workspace,
                         void* stream);
-/* Number of kernels one forward launches (for bench.py's gpu_launches). */
+/* Number of kernels one forward at the batch size of the last forward launches, copies not counted
+ * (for bench.py's gpu_launches). */
 int thmr_engine_num_launches(const thmr_engine* e);
 /* Timed replay for roofline accounting: the forward is a list of launch groups ("steps"); this runs one
  * forward with a CUDA event between steps (synchronises the stream at the end) and returns per-step

@@ -231,6 +231,32 @@ def test_concurrent_engine_matches_default_engine_at_bs64(cuda_dev, tiny):
     assert model.num_launches() == conc.num_launches()
 
 
+@pytest.mark.parametrize("strict", [False, True])
+def test_num_launches_counts_the_kernels_of_a_forward(cuda_dev, strict):
+    """num_launches() is the number of kernels one forward at the last batch size launches, copies not counted.  The
+    SMPL tail runs one blend GEMM and one skinning kernel per 512 poses, so B = 513 launches two more than B = 64."""
+    from torch.profiler import ProfilerActivity, profile
+    from tokenhmr_b200 import synth
+    from tokenhmr_b200.config import tiny_config
+    from tokenhmr_b200.engine import TokenHMREngine
+    cfg = tiny_config(vit_depth=2)
+    model = TokenHMREngine(cfg, synth.make_state_dict(cfg), synth.make_smpl(cfg), device=cuda_dev, max_batch=513,
+                           use_cuda_graph=False, strict=strict, max_cached_shapes=1)
+    n = {}
+    for B in (2, 64, 513):
+        model({"img": synth.make_images(B, cfg, seed=B)})      # builds the plans for B and configures the kernels
+        n[B] = model.num_launches()
+        st = model._state(B, False)
+        torch.cuda.synchronize()
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            model._launch(st, B)
+            torch.cuda.synchronize()
+        kernels = [e.name for e in prof.events() if e.device_type == torch.autograd.DeviceType.CUDA
+                   and "Memcpy" not in e.name and "Memset" not in e.name]
+        assert len(kernels) == n[B], (B, len(kernels), n[B])
+    assert n[513] == n[64] + 2, n
+
+
 def test_release_forward_vs_reference_golden(cuda_dev, golden_dir):
     """Full ViT-H/16 depth-32 forward (B=2) against the outputs of the LIVE reference modules (fp32)."""
     from tokenhmr_b200 import synth

@@ -36,6 +36,17 @@ struct Step {
   const char* name;
   double flops;   // algorithmic FLOPs (2*MAC) of tensor-core work, 0 for bandwidth-bound kernels
   double bytes;   // algorithmic HBM bytes for bandwidth-bound kernels, 0 otherwise
+  int kernels;    // kernels fn launches (copies and memsets not counted): thmr_engine_num_launches
+};
+
+// Appends the steps of one build; tag() sets the label and work recorded with the steps pushed after it.
+struct StepList {
+  std::vector<Step>& v;
+  const char* name = "";
+  double flops = 0, bytes = 0;
+  void tag(const char* n, double f = 0, double b = 0) { name = n; flops = f; bytes = b; }
+  void push_back(StepFn fn, int kernels = 1) { v.push_back(Step{std::move(fn), name, flops, bytes, kernels}); }
+  size_t size() const { return v.size(); }
 };
 
 // ---- SMPL stage (shared by thmr_lbs / thmr_smpl_forward / the engine) -----------------------------------
@@ -65,7 +76,7 @@ inline int smpl_blend_plan(const SmplModel& m, const SmplWs& ws, int p0, int n, 
   d.M = n; d.N = static_cast<int>(ws.off_pitch); d.K = 3 * kSmplPFPad;
   d.out32 = ws.offsets; d.ld32 = static_cast<int>(ws.off_pitch);
   d.alpha = 1.0f / (kSplitScale * kSplitScale);
-  d.force_2cta = 0;
+  d.no_2cta = true;
   return gemm_make_plan(d, plan);
 }
 
@@ -126,7 +137,6 @@ struct thmr_engine {
   int B = 0;
   std::vector<thmr::Step> steps;
   size_t vit_steps = 0;  // steps [0, vit_steps) = backbone
-  int launches = 0;      // kernels per forward (strict mode counts them while building; 0 = default-path formula)
   unsigned long long* stamps = nullptr;   // [kMaxStamps] in the workspace: start stamp of step i, end stamp at [n_steps]
 };
 
@@ -135,6 +145,56 @@ constexpr int kMaxStamps = 2048;
 namespace thmr {
 
 constexpr int kTokPad = 3;  // zero rows on both ends of every tokenizer-decoder sequence (max dilation)
+
+// Workspace of the forward's tail: where the outputs a caller leaves null (thmr_outputs) are written, and SMPL's.
+struct TailWs {
+  float *rot, *betas, *cam, *camt, *focal, *kp3, *kp2, *verts;
+  SmplWs smpl;
+};
+inline void tail_carve(Bump& bp, const SmplModel& m, int B, TailWs* t) {
+  const int NJ = 25 + m.n_extra;
+  t->rot = bp.take<float>(static_cast<size_t>(B) * 24 * 9);
+  t->betas = bp.take<float>(static_cast<size_t>(B) * 16);
+  t->cam = bp.take<float>(static_cast<size_t>(B) * 4);
+  t->camt = bp.take<float>(static_cast<size_t>(B) * 4);
+  t->focal = bp.take<float>(static_cast<size_t>(B) * 2);
+  t->kp3 = bp.take<float>(static_cast<size_t>(B) * NJ * 3);
+  t->kp2 = bp.take<float>(static_cast<size_t>(B) * NJ * 2);
+  t->verts = bp.take<float>(static_cast<size_t>(B) * m.V * 3);
+  smpl_carve(bp, m, B, &t->smpl);
+}
+
+// Read-out assembly, 6D -> rotation (token_head.py:103-128), SMPL + projection (tokenhmr.py:162-187) as one step:
+// readout fp32 [B, 32], out6 fp32 [B, tok_joints + 2 * kTokPad, 8].  The blend GEMM plans are built here.
+inline int add_tail_step(StepList& S, const thmr_engine* e, int B, const TailWs& t, const float* readout,
+                         const float* out6) {
+  const thmr_smpl* sm = e->smpl;
+  const int chunks = (B + kSmplChunk - 1) / kSmplChunk;
+  std::vector<GemmPlan> blend(chunks);
+  for (int ci = 0; ci < chunks; ++ci) {
+    const int p0 = ci * kSmplChunk;
+    THMR_TRY(smpl_blend_plan(sm->m, t.smpl, p0, (B - p0) < kSmplChunk ? (B - p0) : kSmplChunk, &blend[ci]));
+  }
+  const float* ip = e->w.init_pose; const float* ib = e->w.init_betas; const float* ic = e->w.init_cam;
+  const int nb = sm->m.nb, Lpj = e->cfg.tok_joints + 2 * kTokPad, PAD = kTokPad;
+  const float focal = e->cfg.focal_length, isz = static_cast<float>(e->cfg.image_size);
+  S.tag("smpl.lbs");
+  S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
+    float* rot = r.out.rotmats ? r.out.rotmats : t.rot;
+    float* bet = r.out.betas ? r.out.betas : t.betas;
+    float* cam = r.out.pred_cam ? r.out.pred_cam : t.cam;
+    head_assemble_kernel<<<(B * 24 + 127) / 128, 128, 0, st>>>(readout, 32, out6, 8, Lpj, PAD, ip, ib, ic, rot, bet, cam,
+                                                              r.out.pose6d, B, nb);
+    THMR_CUDA(cudaGetLastError());
+    float* verts = r.out.pred_vertices ? r.out.pred_vertices : t.verts;
+    float* kp3 = r.out.pred_keypoints_3d ? r.out.pred_keypoints_3d : t.kp3;
+    float* kp2 = r.out.pred_keypoints_2d ? r.out.pred_keypoints_2d : t.kp2;
+    float* camt = r.out.pred_cam_t ? r.out.pred_cam_t : t.camt;
+    float* foc = r.out.focal_length ? r.out.focal_length : t.focal;
+    return smpl_run(sm, rot, 0, bet, B, verts, nullptr, kp3, cam, focal, isz, camt, foc, kp2, t.smpl, blend.data(), st);
+  }, 3 + 2 * chunks);   // head assemble, pose, per chunk blend GEMM + skin, joints
+  return THMR_OK;
+}
 
 inline size_t engine_build(thmr_engine* e, void* workspace, int B, bool build, int* status, cudaStream_t stream) {
   const thmr_config& c = e->cfg;
@@ -189,30 +249,14 @@ inline size_t engine_build(thmr_engine* e, void* workspace, int B, bool build, i
   const int Lj = c.tok_joints, Lpj = Lj + 2 * PAD;
   float* x32 = bp.take<float>(static_cast<size_t>(B) * Lpj * W);
   float* out6 = bp.take<float>(static_cast<size_t>(B) * Lpj * 8);
-  float* rot_fb = bp.take<float>(static_cast<size_t>(B) * 24 * 9);
-  float* betas_fb = bp.take<float>(static_cast<size_t>(B) * 16);
-  float* cam_fb = bp.take<float>(static_cast<size_t>(B) * 4);
-  float* camt_fb = bp.take<float>(static_cast<size_t>(B) * 4);
-  float* focal_fb = bp.take<float>(static_cast<size_t>(B) * 2);
-  const int NJ = 25 + e->smpl->m.n_extra;
-  float* kp3_fb = bp.take<float>(static_cast<size_t>(B) * NJ * 3);
-  float* kp2_fb = bp.take<float>(static_cast<size_t>(B) * NJ * 2);
-  float* verts_fb = bp.take<float>(static_cast<size_t>(B) * e->smpl->m.V * 3);
-  SmplWs sws;
-  smpl_carve(bp, e->smpl->m, B, &sws);
+  TailWs tail;
+  tail_carve(bp, e->smpl->m, B, &tail);
   const size_t total = (bp.off + 1023) & ~size_t(1023);
   if (!build) return total;
 
   // ---------------------------------------------------------------- steps
   e->steps.clear();
-  struct StepList {
-    std::vector<Step>& v;
-    const char* name = "";
-    double flops = 0, bytes = 0;
-    void tag(const char* n, double f = 0, double b = 0) { name = n; flops = f; bytes = b; }
-    void push_back(StepFn fn) { v.push_back(Step{std::move(fn), name, flops, bytes}); }
-    size_t size() const { return v.size(); }
-  } S{e->steps};
+  StepList S{e->steps};
   int err = THMR_OK;
   e->stamps = stamps;
   auto slot = [&]() -> unsigned long long* { return S.size() < static_cast<size_t>(kMaxStamps - 1) ? stamps + S.size() : nullptr; };
@@ -427,33 +471,8 @@ inline size_t engine_build(thmr_engine* e, void* workspace, int B, bool build, i
   conv(bufA, Lcur, W, w.conv_post, W, 1, 3, kActNone, 0, nullptr, 0, bufB, nullptr);
   conv(bufB, Lcur, W, w.conv_out, 6, 1, 3, kActNone, 0, out6, 8, nullptr, nullptr);
 
-  S.tag("smpl.lbs");
-  // ---- read-out assembly, 6D -> rotation (token_head.py:103-128), SMPL + projection (tokenhmr.py:162-187)
-  {
-    const float* ip = w.init_pose; const float* ib = w.init_betas; const float* ic = w.init_cam;
-    const int nb = e->smpl->m.nb;
-    const thmr_smpl* sm = e->smpl;
-    std::vector<GemmPlan> blend((B + kSmplChunk - 1) / kSmplChunk);
-    for (int ci = 0, p0 = 0; p0 < B; p0 += kSmplChunk, ++ci) {
-      const int s = smpl_blend_plan(sm->m, sws, p0, (B - p0) < kSmplChunk ? (B - p0) : kSmplChunk, &blend[ci]);
-      if (s != THMR_OK) err = s;
-    }
-    const float focal = c.focal_length, isz = static_cast<float>(c.image_size);
-    S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
-      float* rot = r.out.rotmats ? r.out.rotmats : rot_fb;
-      float* bet = r.out.betas ? r.out.betas : betas_fb;
-      float* cam = r.out.pred_cam ? r.out.pred_cam : cam_fb;
-      head_assemble_kernel<<<(B * 24 + 127) / 128, 128, 0, st>>>(readout, 32, out6, 8, Lpj, PAD, ip, ib, ic, rot, bet, cam,
-                                                                r.out.pose6d, B, nb);
-      THMR_CUDA(cudaGetLastError());
-      float* verts = r.out.pred_vertices ? r.out.pred_vertices : verts_fb;
-      float* kp3 = r.out.pred_keypoints_3d ? r.out.pred_keypoints_3d : kp3_fb;
-      float* kp2 = r.out.pred_keypoints_2d ? r.out.pred_keypoints_2d : kp2_fb;
-      float* camt = r.out.pred_cam_t ? r.out.pred_cam_t : camt_fb;
-      float* foc = r.out.focal_length ? r.out.focal_length : focal_fb;
-      return smpl_run(sm, rot, 0, bet, B, verts, nullptr, kp3, cam, focal, isz, camt, foc, kp2, sws, blend.data(), st);
-    });
-  }
+  const int s = add_tail_step(S, e, B, tail, readout, out6);
+  if (s != THMR_OK) err = s;
   *status = err;
   // zero the padded fp16 probability buffer once (pad rows are never written afterwards)
   if (err == THMR_OK) {

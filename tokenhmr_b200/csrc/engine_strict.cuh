@@ -70,74 +70,36 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
   float* bufA = bp.take<float>(static_cast<size_t>(B) * Lp0 * W);
   float* bufB = bp.take<float>(static_cast<size_t>(B) * Lp0 * W);
   float* out6 = bp.take<float>(static_cast<size_t>(B) * Lpj * 8);
-  float* rot_fb = bp.take<float>(static_cast<size_t>(B) * 24 * 9);
-  float* betas_fb = bp.take<float>(static_cast<size_t>(B) * 16);
-  float* cam_fb = bp.take<float>(static_cast<size_t>(B) * 4);
-  float* camt_fb = bp.take<float>(static_cast<size_t>(B) * 4);
-  float* focal_fb = bp.take<float>(static_cast<size_t>(B) * 2);
-  const int NJ = 25 + e->smpl->m.n_extra;
-  float* kp3_fb = bp.take<float>(static_cast<size_t>(B) * NJ * 3);
-  float* kp2_fb = bp.take<float>(static_cast<size_t>(B) * NJ * 2);
-  float* verts_fb = bp.take<float>(static_cast<size_t>(B) * e->smpl->m.V * 3);
-  SmplWs sws;
-  smpl_carve(bp, e->smpl->m, B, &sws);
+  TailWs tail;
+  tail_carve(bp, e->smpl->m, B, &tail);
   const size_t total = (bp.off + 1023) & ~size_t(1023);
   if (!build) return total;
 
   // ---------------------------------------------------------------- steps
   e->steps.clear();
   e->stamps = nullptr;       // (in-graph stamps are a default-mode instrument)
-  struct StepList {
-    std::vector<Step>& v;
-    const char* name = "";
-    double flops = 0, bytes = 0;
-    void tag(const char* n, double f = 0, double b = 0) { name = n; flops = f; bytes = b; }
-    void push_back(StepFn fn) { v.push_back(Step{std::move(fn), name, flops, bytes}); }
-    size_t size() const { return v.size(); }
-  } S{e->steps};
+  StepList S{e->steps};
   int err = THMR_OK;
-  int launches = 0;
 
-  // split(A32) + GEMM over K' = 3K.  `rows` = GEMM M; (sT, spitch, slo) = optional padded-sequence remap of the split;
-  // conv: taps > 1 reads A' rows shifted by tap_row0 + t * tap_stride (A' row = [hi | lo | hi] of cin channels).
-  struct SL {
-    const float* A; long lda; long rows; int K; int act_in;
-    int sT = 0, spitch = 0, slo = 0; long split_rows = 0;     // split_rows: source rows when remapped (else = rows)
-    const void* Wt; int N; const float* bias = nullptr;
-    float* o32; int ld32; const float* resid = nullptr; int ldr = 0; int resid_mod = 0;
-    int taps = 1, dil = 1; int seq_pitch = 0, seq_lo = 0, seq_hi = 0;
-  };
-  auto slinear = [&](const SL& a) {
-    GemmDesc d;
-    d.A = sA; d.lda = 3 * a.K; d.a_rows = a.rows;
-    d.B = static_cast<const __half*>(a.Wt); d.ldb = a.taps * 3 * a.K;
-    d.M = static_cast<int>(a.rows); d.N = a.N; d.K = a.taps * 3 * a.K;
-    d.bias = a.bias; d.resid = a.resid; d.ldr = a.ldr; d.resid_mod = a.resid_mod;
-    d.out32 = a.o32; d.ld32 = a.ld32;
-    d.alpha = kStrictAlpha;
-    if (a.taps > 1) { d.taps = a.taps; d.cin = 3 * a.K; d.tap_row0 = -a.dil; d.tap_stride = a.dil; }
-    d.seq_pitch = a.seq_pitch; d.seq_lo = a.seq_lo; d.seq_hi = a.seq_hi;
-    if (!c.concurrent && gemm_sk_flag_count(a.rows, a.N) <= n_skf) d.sk_flags = skf;
+  // One step of two kernels: split_rows(act_in(A)) of `srows` rows of K channels into sA, then the GEMM d over sA
+  // (split_gemm_desc).  (sT, spitch, slo): optional remap of the split rows into padded sequences (split_rows_kernel).
+  auto slinear = [&](GemmDesc d, const float* A, long lda, long srows, int K, int act_in, int sT = 0, int spitch = 0,
+                     int slo = 0) {
+    if (!c.concurrent && gemm_sk_flag_count(d.M, d.N) <= n_skf) d.sk_flags = skf;
     GemmPlan plan;
     const int s = gemm_make_plan(d, &plan);
     if (s != THMR_OK) { err = s; return; }
-    S.flops = 2.0 * a.rows * a.N * a.taps * a.K;     // algorithmic (one product), the kernel does three
+    S.flops = 2.0 * d.M * d.N * d.taps * K;     // algorithmic (one product), the kernel does three
     S.bytes = 0;
-    const float* A = a.A; const long lda = a.lda; const int K = a.K, act = a.act_in, sT = a.sT, sp = a.spitch, slo = a.slo;
-    const long srows = a.split_rows ? a.split_rows : a.rows;
     __half* dst = sA;
     S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
-      THMR_TRY(split_rows_launch(A, lda, dst, srows, K, act, sT, sp, slo, st));
+      THMR_TRY(split_rows_launch(A, lda, dst, srows, K, act_in, sT, spitch, slo, st));
       return gemm_launch(plan, st);
-    });
-    launches += 2;
+    }, 2);
   };
   auto lin = [&](const float* A, int K, long rows, int act_in, const void* Wt, int N, const float* bias, float* o32,
                  const float* resid = nullptr) {
-    SL a{};
-    a.A = A; a.lda = K; a.rows = rows; a.K = K; a.act_in = act_in; a.Wt = Wt; a.N = N; a.bias = bias; a.o32 = o32; a.ld32 = N;
-    a.resid = resid; a.ldr = N;
-    slinear(a);
+    slinear(split_gemm_desc(sA, rows, K, 1, 1, Wt, N, bias, resid, o32, N), A, K, rows, K, act_in);
   };
   auto ln = [&](const float* in, const float* g, const float* b, float* o32, int R, int C, float eps, int relu, int out_t) {
     S.flops = 0;
@@ -145,15 +107,13 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
       return layernorm_launch(in, g, b, nullptr, 0, o32, R, C, eps, relu, out_t, st);
     });
-    launches += 1;
   };
-  auto push1 = [&](StepFn fn) { S.push_back(std::move(fn)); launches += 1; };
 
   // ---- ViT backbone (vit.py:320-343)
   {
     const int S_ = c.image_size, x0 = (c.image_size - c.crop_w) / 2, Wc = c.crop_w, P = c.patch, pad = c.patch_pad;
     S.tag("vit.patch_im2col", 0, static_cast<double>(B) * 3 * c.image_size * c.crop_w * 4 + static_cast<double>(M) * KP * 4);
-    push1([=](const RunCtx& r, cudaStream_t st) -> int {
+    S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
       const long total_t = static_cast<long>(B) * gh * gw * 3 * P;
       im2col_patch_f32_kernel<<<static_cast<unsigned>((total_t + 255) / 256), 256, 0, st>>>(r.img, a0, B, S_, x0, Wc, P,
                                                                                            pad, gh, gw);
@@ -161,10 +121,9 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
       return THMR_OK;
     });
     S.tag("vit.patch_embed_gemm");
-    SL a{};
-    a.A = a0; a.lda = KP; a.rows = M; a.K = KP; a.Wt = w.patch_w; a.N = D; a.bias = w.patch_b; a.o32 = x; a.ld32 = D;
-    a.resid = w.pos; a.ldr = D; a.resid_mod = T;
-    slinear(a);
+    GemmDesc d = split_gemm_desc(sA, M, KP, 1, 1, w.patch_w, D, w.patch_b, w.pos, x, D);
+    d.resid_mod = T;
+    slinear(d, a0, KP, M, KP, kSplitActNone);
   }
   const float att_scale = 1.0f / sqrtf(static_cast<float>(D / H));
   for (int i = 0; i < c.vit_depth; ++i) {
@@ -174,7 +133,9 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     S.tag("vit.qkv_gemm");
     lin(xn, D, M, kSplitActNone, bw.qkv_w, 3 * D, bw.qkv_b, qkv);
     S.tag("vit.attention", 4.0 * B * H * 192.0 * 192.0 * 80.0, 4.0 * M * D * 4);
-    push1([=](const RunCtx&, cudaStream_t st) -> int { return attention_f32_launch(qkv, 3 * D, B, H, ao, D, att_scale, st); });
+    S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
+      return attention_f32_launch(qkv, 3 * D, B, H, ao, D, att_scale, st);
+    });
     S.tag("vit.proj_gemm");
     lin(ao, D, M, kSplitActNone, bw.proj_w, D, bw.proj_b, x, x);
     S.tag("vit.layernorm");
@@ -188,7 +149,7 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     S.tag("vit.layernorm", 0, static_cast<double>(M) * D * 8);
     const float* g = w.last_g; const float* b = w.last_b;
     const float eps = c.vit_ln_eps;
-    push1([=](const RunCtx& r, cudaStream_t st) -> int {
+    S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
       THMR_TRY(layernorm_launch(x, g, b, nullptr, 0, feat, M, D, eps, 0, 0, st));
       float* t32 = r.vit_tokens_only ? r.vit_tokens_only : r.out.vit_tokens;
       if (t32) THMR_CUDA(cudaMemcpyAsync(t32, feat, sizeof(float) * M * D, cudaMemcpyDeviceToDevice, st));
@@ -203,7 +164,7 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
   S.tag("dec.token_ops");
   {
     const float* t0 = w.token0;
-    push1([=](const RunCtx&, cudaStream_t st) -> int {
+    S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
       broadcast_row_kernel<<<(B * E + 255) / 256, 256, 0, st>>>(t0, tok, B, E);
       THMR_CUDA(cudaGetLastError());
       return THMR_OK;
@@ -219,7 +180,7 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     {
       const int ld = L * 2 * inner, koff = l * 2 * inner, voff = koff + inner, heads = c.dec_heads;
       const float scale = 1.0f / sqrtf(static_cast<float>(c.dec_dim_head));
-      push1([=](const RunCtx&, cudaStream_t st) -> int {
+      S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
         dec_cross_attn_f32_kernel<192><<<B * heads, 192, 0, st>>>(q32, kv, ld, koff, voff, scale, att32, heads);
         THMR_CUDA(cudaGetLastError());
         return THMR_OK;
@@ -230,12 +191,11 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     lin(y32, E, B, kSplitActNone, dw.ff1_w, c.dec_mlp_dim, dw.ff1_b, hid32);
     lin(hid32, c.dec_mlp_dim, B, kSplitActGelu, dw.ff2_w, E, dw.ff2_b, tok, tok);
   }
-  push1([=](const RunCtx& r, cudaStream_t st) -> int {
+  S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
     if (r.out.token_out)
       THMR_CUDA(cudaMemcpyAsync(r.out.token_out, tok, sizeof(float) * B * E, cudaMemcpyDeviceToDevice, st));
     return THMR_OK;
-  });
-  launches -= 1;   // (a memcpy node, not a kernel)
+  }, 0);
   lin(tok, E, B, kSplitActNone, w.readout_w, 32, w.readout_b, readout);
 
   // ---- token classifier (token_classifier.py:89-104)
@@ -247,7 +207,7 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
     ln(cx, mw.ln1_g, mw.ln1_b, yT, B * TN, CH, c.ln_eps, 0, TN);                      // transposed: (B*H, T)
     lin(yT, TN, static_cast<long>(B) * CH, kSplitActNone, mw.tok1_w, c.cls_token_inter, mw.tok1_b, t1);
     lin(t1, c.cls_token_inter, static_cast<long>(B) * CH, kSplitActGelu, mw.tok2_w, TN, mw.tok2_b, yT2);
-    push1([=](const RunCtx&, cudaStream_t st) -> int {
+    S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
       const long n = static_cast<long>(B) * TN * CH;
       mixer_add_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(cx, yT2, nullptr, xy, B, TN, CH);
       THMR_CUDA(cudaGetLastError());
@@ -269,35 +229,26 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
       THMR_CUDA(cudaMemcpyAsync(probs_fallback, p32, sizeof(float) * B * TN * NC, cudaMemcpyDeviceToDevice, st));
     return THMR_OK;
   });
-  launches += 1;
 
   S.tag("tok.decoder_ops");
   // ---- tokenizer: soft codebook lookup + Conv1d decoder (vanilla_pose_vqvae.py:294-297, 135-154)
-  {
-    SL a{};   // dequantize_logits on the padded layout: the split scatters the B*TN rows into [B, Lp0] sequences; the
-              // pad rows of the scratch hold stale data, so the output rows are masked to zero (real zeros for the conv)
-    a.A = probs_fallback; a.lda = NC; a.rows = static_cast<long>(B) * Lp0; a.split_rows = static_cast<long>(B) * TN;
-    a.K = NC; a.act_in = kSplitActNone; a.sT = TN; a.spitch = Lp0; a.slo = PAD;
-    a.Wt = w.codebook_t; a.N = c.code_dim; a.o32 = d32; a.ld32 = c.code_dim;
-    a.seq_pitch = Lp0; a.seq_lo = PAD; a.seq_hi = PAD + TN;
-    slinear(a);
-  }
+  // dequantize_logits on the padded layout: the split scatters the B*TN rows into [B, Lp0] sequences; the pad rows of
+  // the scratch hold stale data, so the output rows are masked to zero (real zeros for the conv)
+  slinear(split_gemm_desc(sA, static_cast<long>(B) * Lp0, NC, 1, 1, w.codebook_t, c.code_dim, nullptr, nullptr, d32,
+                          c.code_dim, TN, PAD),
+          probs_fallback, NC, static_cast<long>(B) * TN, NC, kSplitActNone, TN, Lp0, PAD);
   auto conv = [&](const float* in, int Lcur, int cin, int act_in, const thmr_conv& cw, int cout, int dil, int taps,
                   float* o32, int ld32, const float* resid) {
-    const int Lp = Lcur + 2 * PAD;
-    SL a{};
-    a.A = in; a.lda = cin; a.rows = static_cast<long>(B) * Lp; a.K = cin; a.act_in = act_in;
-    a.Wt = cw.w; a.N = cout; a.bias = cw.b; a.o32 = o32; a.ld32 = ld32; a.resid = resid; a.ldr = ld32;
-    a.taps = taps; a.dil = dil;
-    a.seq_pitch = Lp; a.seq_lo = PAD; a.seq_hi = PAD + Lcur;
-    slinear(a);
+    const long rows = static_cast<long>(B) * (Lcur + 2 * PAD);
+    slinear(split_gemm_desc(sA, rows, cin, taps, dil, cw.w, cout, cw.b, resid, o32, ld32, Lcur, PAD), in, cin, rows, cin,
+            act_in);
   };
   int Lcur = TN;
   // activations are applied by the consumer's split: bufA holds the PRE-ReLU conv output from here on
   conv(d32, Lcur, c.code_dim, kSplitActNone, w.conv_in, W, 1, 3, bufA, W, nullptr);
   for (int u = 0; u < c.n_upsample; ++u) {
     const int Lout = c.upsample_sizes[u], Lin = Lcur;
-    push1([=](const RunCtx&, cudaStream_t st) -> int {      // nearest gather commutes with ReLU: copy the pre-ReLU rows
+    S.push_back([=](const RunCtx&, cudaStream_t st) -> int {   // nearest gather commutes with ReLU: copy the pre-ReLU rows
       const long n = static_cast<long>(B) * (Lout + 2 * PAD) * (W / 4);
       upsample_rows_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(
           reinterpret_cast<const __half*>(bufA), reinterpret_cast<__half*>(bufB), B, Lin, Lout, PAD, W / 4);
@@ -312,7 +263,7 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
   float* xres = bufA;
   {
     const long n4 = static_cast<long>(B) * (Lcur + 2 * PAD) * W / 4;
-    push1([=](const RunCtx&, cudaStream_t st) -> int {
+    S.push_back([=](const RunCtx&, cudaStream_t st) -> int {
       relu_inplace_kernel<<<static_cast<unsigned>((n4 + 255) / 256), 256, 0, st>>>(xres, n4);
       THMR_CUDA(cudaGetLastError());
       return THMR_OK;
@@ -327,34 +278,8 @@ inline size_t engine_build_strict(thmr_engine* e, void* workspace, int B, bool b
   conv(xres, Lcur, W, kSplitActNone, w.conv_post, W, 1, 3, bufB, W, nullptr);
   conv(bufB, Lcur, W, kSplitActNone, w.conv_out, 6, 1, 3, out6, 8, nullptr);
 
-  S.tag("smpl.lbs");
-  {
-    const float* ip = w.init_pose; const float* ib = w.init_betas; const float* ic = w.init_cam;
-    const int nb = e->smpl->m.nb;
-    const thmr_smpl* sm = e->smpl;
-    std::vector<GemmPlan> blend((B + kSmplChunk - 1) / kSmplChunk);
-    for (int ci = 0, p0 = 0; p0 < B; p0 += kSmplChunk, ++ci) {
-      const int s = smpl_blend_plan(sm->m, sws, p0, (B - p0) < kSmplChunk ? (B - p0) : kSmplChunk, &blend[ci]);
-      if (s != THMR_OK) err = s;
-    }
-    const float focal = c.focal_length, isz = static_cast<float>(c.image_size);
-    S.push_back([=](const RunCtx& r, cudaStream_t st) -> int {
-      float* rot = r.out.rotmats ? r.out.rotmats : rot_fb;
-      float* bet = r.out.betas ? r.out.betas : betas_fb;
-      float* cam = r.out.pred_cam ? r.out.pred_cam : cam_fb;
-      head_assemble_kernel<<<(B * 24 + 127) / 128, 128, 0, st>>>(readout, 32, out6, 8, Lpj, PAD, ip, ib, ic, rot, bet, cam,
-                                                                r.out.pose6d, B, nb);
-      THMR_CUDA(cudaGetLastError());
-      float* verts = r.out.pred_vertices ? r.out.pred_vertices : verts_fb;
-      float* kp3 = r.out.pred_keypoints_3d ? r.out.pred_keypoints_3d : kp3_fb;
-      float* kp2 = r.out.pred_keypoints_2d ? r.out.pred_keypoints_2d : kp2_fb;
-      float* camt = r.out.pred_cam_t ? r.out.pred_cam_t : camt_fb;
-      float* foc = r.out.focal_length ? r.out.focal_length : focal_fb;
-      return smpl_run(sm, rot, 0, bet, B, verts, nullptr, kp3, cam, focal, isz, camt, foc, kp2, sws, blend.data(), st);
-    });
-    launches += 5;
-  }
-  e->launches = launches;
+  const int s = add_tail_step(S, e, B, tail, readout, out6);
+  if (s != THMR_OK) err = s;
   *status = err;
   if (err == THMR_OK && cudaMemsetAsync(skf, 0, n_skf * sizeof(unsigned), stream) != cudaSuccess)
     *status = fail(THMR_ERR_CUDA, "cudaMemsetAsync(stream-K flags) failed");

@@ -34,9 +34,8 @@ struct GemmDesc {
   int* screen_rows = nullptr; int* screen_count = nullptr; const float* screen_cmax2 = nullptr;
   float screen_rel = 0.f, screen_abs = 0.f; int screen_row0 = 0;
   const int* row_map = nullptr; const int* m_dev = nullptr; int m_dev_off = 0;
-  int force_bn = 0;
-  int force_epi = -1;  // 0 forces the generic epilogue (tests)
-  int force_2cta = -1; // -1 auto, 0 never, 1 always (when eligible)
+  int force_bn = 0;      // 512: the CTA-pair kernel whatever the shape (needs a TMA epilogue)
+  bool no_2cta = false;  // never use the CTA-pair kernel
   unsigned int* sk_flags = nullptr;  // >= gemm_sk_flag_count(M, N) zeroed uints: enables stream-K for reduce-add GEMMs
   unsigned long long* stamp = nullptr;   // in-graph start stamp slot (nullable)
 };
@@ -108,7 +107,6 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
   int epi = pick_epi(d);
   if (d.force_bn && d.force_bn < 128) epi = kEpiGeneric;
   THMR_CHECK(d.force_bn != 512 || epi != kEpiGeneric, "gemm: block_n 512 (CTA pair) needs a TMA-epilogue eligible call");
-  if (d.force_epi >= 0) epi = d.force_epi == kEpiGeneric ? kEpiGeneric : epi;
   const int bn = pick_bn(d.M, d.N, d.force_bn == 512 ? 0 : d.force_bn, epi);
   THMR_CHECK(bn == 32 || bn == 64 || bn == 128 || bn == 256, "gemm: bad block_n %d", bn);
   GemmParams& p = plan->p;
@@ -136,9 +134,8 @@ inline int gemm_make_plan(const GemmDesc& d, GemmPlan* plan) {
     p.kblocks_per_tap = num_kb;
   }
   // CTA-pair kernel for the large TMA-epilogue GEMMs (the ViT projections)
-  bool two = epi != kEpiGeneric && d.taps == 1 && d.M >= 256 && d.N >= 256 && !d.force_bn;
-  if (d.force_2cta == 0) two = false;
-  if (d.force_2cta == 1 || d.force_bn == 512) two = epi != kEpiGeneric && d.taps == 1;
+  const bool two = epi != kEpiGeneric && d.taps == 1 && !d.no_2cta &&
+                   (d.force_bn == 512 || (d.M >= 256 && d.N >= 256 && !d.force_bn));
   plan->two_cta = two ? 1 : 0;
   THMR_TRY(make_tmap_2d_f16(&plan->tmA, d.A, d.a_rows, a_cols, d.lda, kGemmBM, kGemmBK, CU_TENSOR_MAP_SWIZZLE_128B));
   const int b_box_rows = two ? kG2BN / 2 : bn;

@@ -16,6 +16,7 @@
 #pragma once
 #include "common.cuh"
 #include "elementwise.cuh"
+#include "gemm_host.cuh"
 
 namespace thmr {
 
@@ -72,6 +73,26 @@ inline int split_rows_launch(const float* src, long lds, __half* dst, long R, in
   split_rows_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, st>>>(src, lds, dst, R, C, act, T, pitch, lo);
   THMR_CUDA(cudaGetLastError());
   return THMR_OK;
+}
+
+// The GEMM over a split operand: sA = split_rows of `rows` rows of K channels, times the split weight f16 [N, taps * 3K]
+// (per tap [hi | hi | lo] of w * 2^8, packed on the host); out32 = 2^-12 * acc + bias (+ resid), both with row pitch
+// ld32.  taps > 1: implicit conv1d, tap t reads row m + (t - 1) * dil.  seq_len > 0: the rows are sequences of seq_len
+// rows with seq_pad zero rows on either side, and the pad rows of the output are written as zero.
+inline GemmDesc split_gemm_desc(const __half* sA, long rows, int K, int taps, int dil, const void* Wt, int N,
+                                const float* bias, const float* resid, float* o32, int ld32, int seq_len = 0,
+                                int seq_pad = 0) {
+  const int ks = 3 * K;   // one split row: [hi | lo | hi]
+  GemmDesc d;
+  d.A = sA; d.lda = ks; d.a_rows = rows;
+  d.B = static_cast<const __half*>(Wt); d.ldb = taps * ks;
+  d.M = static_cast<int>(rows); d.N = N; d.K = taps * ks;
+  d.bias = bias; d.resid = resid; d.ldr = ld32;
+  d.out32 = o32; d.ld32 = ld32;
+  d.alpha = kStrictAlpha;
+  if (taps > 1) { d.taps = taps; d.cin = ks; d.tap_row0 = -dil; d.tap_stride = dil; }
+  if (seq_len > 0) { d.seq_pitch = seq_len + 2 * seq_pad; d.seq_lo = seq_pad; d.seq_hi = seq_pad + seq_len; }
+  return d;
 }
 
 __global__ void relu_inplace_kernel(float* __restrict__ x, long n4) {

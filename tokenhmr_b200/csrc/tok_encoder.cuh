@@ -102,25 +102,15 @@ inline void enc_carve(const thmr_tok_encoder_desc& d, void* base, int B, EncWs* 
   ws->total = (bp.off + 1023) & ~size_t(1023);
 }
 
-// One convolution in split precision: A' = split(act_in(in32)) [rows, 3*cin], weight f16 [cout, taps*3*cin] (per tap
-// [hi | hi | lo], packed by tokenizer.py), out32 = alpha * acc + bias (+ resid), pad rows of the output zero.
+// One convolution in split precision: split(act_in(in32)) into sA, then out32 = conv(., weight) + bias (+ resid) with
+// the pad rows of the output zero (split_gemm_desc; the weights are packed by tokenizer.py).
 inline int enc_conv(const float* in, int B, int Lcur, int cin, int taps, int dil, int act_in, const thmr_tok_conv& cw,
                     int cout, float* o32, const float* resid, __half* sA, cudaStream_t st) {
-  const int Lp = Lcur + 2 * kEncPad;
-  const long rows = static_cast<long>(B) * Lp;
+  const long rows = static_cast<long>(B) * (Lcur + 2 * kEncPad);
   THMR_TRY(split_rows_launch(in, cin, sA, rows, cin, act_in, 0, 0, 0, st));
-  GemmDesc d;
-  d.A = sA; d.lda = 3 * cin; d.a_rows = rows;
-  d.B = static_cast<const __half*>(cw.w); d.ldb = taps * 3 * cin;
-  d.M = static_cast<int>(rows); d.N = cout; d.K = taps * 3 * cin;
-  d.bias = cw.b;
-  d.resid = resid; d.ldr = cout;
-  d.out32 = o32; d.ld32 = cout;
-  d.alpha = kStrictAlpha;
-  if (taps > 1) { d.taps = taps; d.cin = 3 * cin; d.tap_row0 = -dil; d.tap_stride = dil; }
-  d.seq_pitch = Lp; d.seq_lo = kEncPad; d.seq_hi = kEncPad + Lcur;
   GemmPlan plan;
-  THMR_TRY(gemm_make_plan(d, &plan));
+  THMR_TRY(gemm_make_plan(split_gemm_desc(sA, rows, cin, taps, dil, cw.w, cout, cw.b, resid, o32, cout, Lcur, kEncPad),
+                          &plan));
   return gemm_launch(plan, st);
 }
 

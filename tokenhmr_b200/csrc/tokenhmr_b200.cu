@@ -715,9 +715,9 @@ int thmr_engine_profile(thmr_engine* e, const float* img, int B, const thmr_outp
 
 int thmr_engine_num_launches(const thmr_engine* e) {
   if (!e) return 0;
-  // every step is one kernel except the SMPL tail (assemble + pose + blend GEMM + skin + joints = 5)
-  if (e->cfg.strict) return e->launches;
-  return e->steps.empty() ? 0 : static_cast<int>(e->steps.size()) + 4;
+  int n = 0;
+  for (const Step& s : e->steps) n += s.kernels;
+  return n;
 }
 
 // ------------------------------------------------------------------------------------------ multi-GPU exchange
